@@ -13,6 +13,7 @@ queries/sec on a 1M-item index) is reported in `knn_summary` (scalars, early in 
 Further keys: `roofline` / `roofline_summary`, `cpu_baseline`, `clocks`, `get_batch_e2e` (host float features in),
 `config0_batch1024`, `mining_regimes` (N=1), `weights_identical_across_ranks`, `strong_scaling` (N>1), `desim`.
   --tower vnet|wide|resnet   --dtype fp16|bf16   --features uniform|clustered   --scaling weak|strong   --no-extras
+  --dump-outputs DIR   after the run, write what the timed paths computed as DIR/<name>.npy (see dump_outputs)
 """
 import argparse
 import json
@@ -57,6 +58,42 @@ def peaks():
     p.update({k: m[k] for k in ("hbm_gbs", "bf16_tflops", "bf16_tflops_sustained") if k in m})
     p["source"] = "measured"
   return p
+
+
+DUMP_SAMPLE_ROWS = 4096             # queries of the KNN result / rows of the de-similarity output
+DUMP_SAMPLE_WEIGHTS = 1 << 22       # elements of the flat weight buffer (VNet has 8.8M, the wide tower 13.1M)
+# the most --dump-outputs writes: the weight sample (fp32), the KNN sample at k=100 (fp32 distances + float64 ids), the
+# de-similarity sample at 81 neighbours (float64) and the 4 training stats -- about 24 MB, fixed by the sizes above
+DUMP_MAX_BYTES = 4 * DUMP_SAMPLE_WEIGHTS + DUMP_SAMPLE_ROWS * (100 * (4 + 8) + 81 * 8) + 4 * 4
+assert DUMP_MAX_BYTES <= 64 << 20
+
+
+def sample_index(n, k, seed=0):
+  """Ascending indices of a fixed, seeded sample of k of n rows (all n when n <= k): the same rows on every run."""
+  if n <= k:
+    return np.arange(n)
+  return np.sort(np.random.RandomState(seed).choice(n, k, replace=False))
+
+
+def sample_rows(t, k):
+  import torch
+  return t[torch.as_tensor(sample_index(t.shape[0], k), device=t.device)].cpu().numpy()
+
+
+def dump_outputs(out_dir, arrays):
+  """What the timed paths computed, one float32 / float64 .npy per array, so that two builds run with the same arguments
+  (hence the same seeded inputs) can be compared output for output:
+    train_stats    [4] stats the last timed training step returned (loss first)
+    train_weights  seeded sample of the flat fp32 weight buffer right after that step
+    knn_distances, knn_ids   seeded sample of query rows of the last timed KNN search (ids as float64, exact)
+    desim_out      seeded sample of rows of the last timed de-similarity filter call (-1 = dropped; float64)
+  The inputs are seeded, so they are the same on every run.  Two runs of one build wrote identical arrays (measured on a
+  B200 at 1000 W).  Across builds the kernels may round differently: compare train_stats, train_weights and knn_distances
+  with a tolerance, the ids and desim_out exactly up to ties."""
+  os.makedirs(out_dir, exist_ok=True)
+  for name, a in arrays.items():
+    assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+    np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler(object):
@@ -188,7 +225,7 @@ def cpu_desim_baseline(budget_s=8.0, n=20000, ke=81, kf=26):
                     "iter_desim_mp; the reference itself spawns 81 x Pool(22) numpy passes) in %.1f s" % (rows, ke, n, kf, dt)}
 
 
-def bench_desim(torch, ops, dev, n, world, rank, barrier, dist, pk, ke=81, kf=26, reps=5):
+def bench_desim(torch, ops, dev, n, world, rank, barrier, dist, pk, ke=81, kf=26, reps=5, dump=None):
   gen = torch.Generator(device=dev)
   gen.manual_seed(6 + rank)
   eI, fI, fD = _desim_inputs(gen, n, ke, kf, torch, dev)
@@ -201,6 +238,8 @@ def bench_desim(torch, ops, dev, n, world, rank, barrier, dist, pk, ke=81, kf=26
     ops.desim(eI, fI, fD, 1.4, 31, out=out)
   e1.record()
   barrier()
+  if dump is not None:
+    dump["desim_out"] = sample_rows(out, DUMP_SAMPLE_ROWS).astype(np.float64)
   t = torch.tensor([e0.elapsed_time(e1) / reps], device=dev, dtype=torch.float64)
   if world > 1:
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -330,8 +369,13 @@ def main():
   ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                   help="weak: --batch triplets per GPU; strong: --batch triplets per step split over the GPUs")
   ap.add_argument("--no-extras", action="store_true", help="skip the secondary measurements (regimes, configs[0], strong scaling)")
+  ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                  help="write what the timed steps computed (last training step, KNN search, de-similarity filter) as "
+                       "DIR/<name>.npy, about 24 MB in all")
   args = ap.parse_args()
   args.warmup = max(args.warmup, 3)
+  if args.dump_outputs and args.impl == "reference":
+    ap.error("--dump-outputs applies to --impl ours")
   if args.impl == "reference":
     return run_reference(args)
 
@@ -446,6 +490,10 @@ def main():
   launches = ops.launch_count() - launches0
   clocks = sampler.stop() if rank == 0 else None
   loss_last = float(stats[0].item())
+  dump = {} if args.dump_outputs else None
+  if dump is not None:                # before the e2e steps below train on
+    dump["train_stats"] = stats.cpu().numpy().astype(np.float32)
+    dump["train_weights"] = sample_rows(eng.w, DUMP_SAMPLE_WEIGHTS)
   t = torch.tensor([ms], device=dev, dtype=torch.float64)
   if world > 1:
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -711,6 +759,9 @@ def main():
       return out, float(np.median(times)), times
 
     (D, I), kms, kms_all = timed_search(5)
+    if dump is not None:
+      dump["knn_distances"] = sample_rows(D, DUMP_SAMPLE_ROWS)
+      dump["knn_ids"] = sample_rows(I, DUMP_SAMPLE_ROWS).astype(np.float64)
     kms_slice, kms_slice_all = None, None
     if world > 1:       # the same search leaving every rank with ITS slice of the queries (no final all-gather)
       _, kms_slice, kms_slice_all = timed_search(5, gather=False)
@@ -772,7 +823,7 @@ def main():
   # ---- SURVEY 8f row 2: de-similarity filter of the KNN lists (integer work, HBM-bound; rows are independent -> each
   # rank filters its own slice of the rows, no collective: weak scaling)
   if not args.no_desim:
-    line["desim"] = bench_desim(torch, ops, dev, args.desim_n, world, rank, barrier, dist, pk)
+    line["desim"] = bench_desim(torch, ops, dev, args.desim_n, world, rank, barrier, dist, pk, dump=dump)
   line["roofline"] = roofline          # last: its per-GEMM list is the long tail of the line
   if world > 1:                       # a teardown that does not finish within a minute must not hold the job
     t = threading.Timer(60.0, os._exit, (0,))
@@ -783,6 +834,8 @@ def main():
       dist.barrier()
       dist.destroy_process_group()
     return
+  if dump is not None:                # rank 0: the weights are identical on every rank
+    dump_outputs(args.dump_outputs, dump)
   if not args.no_cpu and world == 1:
     if not args.no_desim:
       line["desim"]["cpu_baseline"] = cpu_desim_baseline()

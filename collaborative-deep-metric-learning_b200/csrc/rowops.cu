@@ -107,11 +107,37 @@ rows_normalize_cast_kernel(const float* __restrict__ in, int64_t n, int64_t F, i
 // ------------------------------------------------------------------------------------------------
 // K5 hinge loss (losses.py:33-38) + gradient
 // ------------------------------------------------------------------------------------------------
-template <bool kScatter>
+// With mined negatives (kMined) several triplets may pick the same negative row, whose gradient is then a sum over those
+// triplets.  Float atomics would make that sum depend on the order the triplets arrive in, so a training step would not
+// be reproducible.  Instead each row's sum of (a - n) is accumulated in 64-bit fixed point -- integer adds are
+// associative -- and added to the row once:
+//   hinge_triplet_kernel<true>  plain stores of the anchor / positive rows (each owned by one triplet), zero rows 3i+2;
+//                               per active triplet: claim the lowest triplet index as the negative row's accumulator
+//                               slot, and the row's largest |a - n| (it fixes the row's fixed-point scale)
+//   hinge_neg_accum_kernel      integer atomics of round((a - n) * 2^k) into the slot's D accumulators
+//   hinge_neg_apply_kernel      per slot: G[n] += s * sum * 2^-k
+// k is chosen per row so that at most 2^log2B terms of magnitude <= the row's largest |a - n| stay below 2^62.
+// Non-finite inputs: a triplet whose distances are NaN has h = fmaxf(NaN, 0) = 0, is inactive and adds nothing to its
+// negative row (its own anchor / positive rows still get 0 * NaN = NaN).  A row that receives a non-finite a - n from an
+// active triplet becomes NaN in every element, where a float sum would give +-inf or NaN in the affected elements only.
+// Either way the optimizer step that follows turns those weights into NaN.
+struct MinedScratch {
+  uint32_t* slot_inv;      // [3B] ~(lowest active triplet that picked the row); 0 = none
+  uint32_t* row_max;       // [3B] bits of the row's largest |a - n| (non-negative floats order as integers; NaN wins)
+  long long* acc;          // [B, D] fixed-point sums, indexed by slot
+};
+
+__device__ __forceinline__ int mined_scale(float m, int log2B) {
+  int e;
+  frexpf(m, &e);           // m < 2^e
+  return 62 - log2B - e;
+}
+
+template <bool kMined>
 __global__ void __launch_bounds__(kRowThreads)
 hinge_triplet_kernel(const float* __restrict__ E, int64_t B, int D, int64_t ld, const int32_t* __restrict__ neg_row,
                      float margin, float gscale, float* __restrict__ pos_dist, float* __restrict__ neg_dist,
-                     float* __restrict__ hinge, float* __restrict__ G) {
+                     float* __restrict__ hinge, float* __restrict__ G, MinedScratch ms) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int64_t i = static_cast<int64_t>(blockIdx.x) * kWarpsPerBlock + warp; i < B;
        i += static_cast<int64_t>(gridDim.x) * kWarpsPerBlock) {
@@ -136,18 +162,75 @@ hinge_triplet_kernel(const float* __restrict__ E, int64_t B, int D, int64_t ld, 
     }
     if (G != nullptr) {
       const float s = h > 0.f ? 2.f * gscale : 0.f;
-      for (int j = lane; j < D; j += 32) {
-        const float av = a[j], pv = p[j], nv = ng[j];
-        const float ga = s * (nv - pv), gp = s * (pv - av), gn = s * (av - nv);
-        if (kScatter) {
-          atomicAdd(G + ra * ld + j, ga);
-          atomicAdd(G + rp * ld + j, gp);
-          atomicAdd(G + rn * ld + j, gn);
-        } else {
-          G[ra * ld + j] = ga, G[rp * ld + j] = gp, G[rn * ld + j] = gn;
+      if (kMined) {
+        uint32_t mx = 0u;
+        for (int j = lane; j < static_cast<int>(ld); j += 32) {
+          float ga = 0.f, gp = 0.f;
+          if (j < D) {
+            const float av = a[j], pv = p[j], nv = ng[j];
+            ga = s * (nv - pv), gp = s * (pv - av);
+            mx = max(mx, __float_as_uint(fabsf(av - nv)));
+          }
+          G[ra * ld + j] = ga, G[rp * ld + j] = gp, G[(3 * i + 2) * ld + j] = 0.f;
+        }
+        mx = __reduce_max_sync(0xffffffffu, mx);
+        if (h > 0.f) {
+          long long* acc = ms.acc + i * D;
+          for (int j = lane; j < D; j += 32) acc[j] = 0;
+          if (lane == 0) {
+            atomicMax(ms.slot_inv + rn, ~static_cast<uint32_t>(i));
+            atomicMax(ms.row_max + rn, mx);
+          }
+        }
+      } else {
+        for (int j = lane; j < D; j += 32) {
+          const float av = a[j], pv = p[j], nv = ng[j];
+          G[ra * ld + j] = s * (nv - pv), G[rp * ld + j] = s * (pv - av), G[rn * ld + j] = s * (av - nv);
         }
       }
     }
+  }
+}
+
+__global__ void __launch_bounds__(kRowThreads)
+hinge_neg_accum_kernel(const float* __restrict__ E, int64_t B, int D, int64_t ld, const int32_t* __restrict__ neg_row,
+                       const float* __restrict__ hinge, MinedScratch ms, int log2B) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int64_t i = static_cast<int64_t>(blockIdx.x) * kWarpsPerBlock + warp; i < B;
+       i += static_cast<int64_t>(gridDim.x) * kWarpsPerBlock) {
+    if (!(hinge[i] > 0.f)) continue;
+    const int64_t rn = neg_row[i];
+    const float m = __uint_as_float(ms.row_max[rn]);
+    if (!(m > 0.f) || !isfinite(m)) continue;              // all zero: nothing to add; not finite: the apply pass writes NaN
+    const int k = mined_scale(m, log2B);
+    unsigned long long* acc = reinterpret_cast<unsigned long long*>(ms.acc + static_cast<int64_t>(~ms.slot_inv[rn]) * D);
+    const float* a = E + 3 * i * ld;
+    const float* ng = E + rn * ld;
+    for (int j = lane; j < D; j += 32)
+      atomicAdd(acc + j, static_cast<unsigned long long>(__float2ll_rn(scalbnf(a[j] - ng[j], k))));
+  }
+}
+
+__global__ void __launch_bounds__(kRowThreads)
+hinge_neg_apply_kernel(int64_t B, int D, int64_t ld, const int32_t* __restrict__ neg_row, const float* __restrict__ hinge,
+                       float gscale, MinedScratch ms, int log2B, float* __restrict__ G) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int64_t i = static_cast<int64_t>(blockIdx.x) * kWarpsPerBlock + warp; i < B;
+       i += static_cast<int64_t>(gridDim.x) * kWarpsPerBlock) {
+    if (!(hinge[i] > 0.f)) continue;
+    const int64_t rn = neg_row[i];
+    if (~ms.slot_inv[rn] != static_cast<uint32_t>(i)) continue;    // one triplet per negative row applies the sum
+    const float m = __uint_as_float(ms.row_max[rn]);
+    if (m == 0.f) continue;
+    const float s = 2.f * gscale;
+    float* g = G + rn * ld;
+    if (!isfinite(m)) {
+      for (int j = lane; j < D; j += 32) g[j] += s * __int_as_float(0x7fc00000);
+      continue;
+    }
+    const int k = mined_scale(m, log2B);
+    const long long* acc = ms.acc + i * D;
+    for (int j = lane; j < D; j += 32) g[j] += s * scalbnf(__ll2float_rn(acc[j]), -k);
   }
 }
 
@@ -623,12 +706,25 @@ int cdml_triplet_hinge(cdml_ctx* ctx, const float* E, int64_t B, int D, int64_t 
                "cdml_triplet_hinge: dz16 needs rinv and an even ld_dz >= D");
   const int grid = row_grid(ctx, B);
   if (neg_row != nullptr && G != nullptr) {
-    CDML_CHECK_CUDA(cudaMemsetAsync(G, 0, sizeof(float) * 3 * B * ld_e, st));
+    CDML_REQUIRE(3 * B < (1ll << 31), "cdml_triplet_hinge: B=%lld too large for mined negatives", (long long)B);
+    // scratch: slot_inv [3B] u32 | row_max [3B] u32 | acc [B, D] i64 (the first two zeroed by one memset)
+    const size_t head = sizeof(uint32_t) * 6 * B;
+    uint8_t* ws = static_cast<uint8_t*>(ctx_scratch(ctx, head + sizeof(long long) * B * D));
+    if (ws == nullptr) return -2;
+    MinedScratch ms{reinterpret_cast<uint32_t*>(ws), reinterpret_cast<uint32_t*>(ws) + 3 * B,
+                    reinterpret_cast<long long*>(ws + head)};
+    int log2B = 0;
+    while ((1ll << log2B) < B) ++log2B;
+    CDML_CHECK_CUDA(cudaMemsetAsync(ws, 0, head, st));
     hinge_triplet_kernel<true><<<grid, kRowThreads, 0, st>>>(E, B, D, ld_e, neg_row, margin, grad_scale, pos_dist,
-                                                            neg_dist, hinge_dist, G);
+                                                            neg_dist, hinge_dist, G, ms);
+    CDML_CHECK_CUDA(cudaGetLastError());
+    hinge_neg_accum_kernel<<<grid, kRowThreads, 0, st>>>(E, B, D, ld_e, neg_row, hinge_dist, ms, log2B);
+    CDML_CHECK_CUDA(cudaGetLastError());
+    hinge_neg_apply_kernel<<<grid, kRowThreads, 0, st>>>(B, D, ld_e, neg_row, hinge_dist, grad_scale, ms, log2B, G);
   } else {
     hinge_triplet_kernel<false><<<grid, kRowThreads, 0, st>>>(E, B, D, ld_e, neg_row, margin, grad_scale, pos_dist,
-                                                             neg_dist, hinge_dist, G);
+                                                             neg_dist, hinge_dist, G, MinedScratch{});
   }
   CDML_CHECK_CUDA(cudaGetLastError());
   hinge_stats_kernel<<<1, 1024, 0, st>>>(hinge_dist, pos_dist, neg_dist, B, stats);

@@ -143,7 +143,8 @@ def triplet_hinge(E, B, margin, neg_row=None, grad_scale=1.0, rinv=None, leaky_a
     dE = out.get("dE") if "dE" in out else torch.empty_like(E)
   if dz16 is not None and dE is None and workspace is None:
     workspace = torch.empty((3 * B * E.stride(0),), dtype=torch.float32, device=dev)
-  _count(2 + (1 if dz16 is not None else 0))
+  mined_grad = neg_row is not None and (dE is not None or dz16 is not None)     # + the two fixed-point passes
+  _count(2 + (2 if mined_grad else 0) + (1 if dz16 is not None else 0))
   check(_lib.load().cdml_triplet_hinge(_ctx(E), ptr(E), B, D, E.stride(0), ptr(neg_row), float(margin), float(grad_scale),
                                        ptr(rinv), float(leaky_alpha), ptr(pos), ptr(neg), ptr(hin), ptr(stats), ptr(dE),
                                        ptr(dz16), dz16.stride(0) if dz16 is not None else 0,

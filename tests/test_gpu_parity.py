@@ -100,6 +100,45 @@ def test_hinge_loss_fixture_and_random(cd):
   assert np.allclose(r["dE"].cpu().numpy(), O.hinge_loss_grad(E, 0.8).reshape(-1, 256), atol=1e-9)
 
 
+@pytest.mark.parametrize("B", [4096, 3001])
+def test_hinge_gradient_with_mined_negatives_is_exact_and_reproducible(cd, B):
+  """Mined negatives alias rows: several triplets pick the same row, here up to 512 of them, on a row 3i+2 (no gradient of
+  its own) and on a positive row.  The gradient equals the float64 sum, and is bit-identical from call to call (the sum
+  over the triplets that picked a row must not depend on the order they are processed in) -- returned as dE, and in the
+  training form, where it lands in the caller's workspace and only the fp16 dz of the L2-norm / leaky backward is kept."""
+  D, margin, alpha = 256, 0.1, 0.2
+  rs = np.random.RandomState(11)
+  E = O.l2_normalize(rs.standard_normal((3 * B, D))).astype(np.float32)
+  neg = (3 * rs.randint(0, B, B) + rs.randint(1, 3, B)).astype(np.int32)        # positives / negatives, as the miner picks
+  neg[:512], neg[512:800] = 5, 7
+  rinv = rs.uniform(0.5, 2.0, 3 * B).astype(np.float32)
+  a, p, n = E[0::3].astype(np.float64), E[1::3].astype(np.float64), E[neg].astype(np.float64)
+  h = np.maximum(((a - p) ** 2).sum(1) - ((a - n) ** 2).sum(1) + margin, 0.0)
+  s = np.where(h > 0, 2.0, 0.0)[:, None]
+  want = np.zeros((3 * B, D))
+  want[0::3], want[1::3] = s * (n - p), s * (p - a)
+  bound = np.abs(want)
+  np.add.at(want, neg, s * (a - n))
+  np.add.at(bound, neg, np.abs(s * (a - n)))
+  E64 = E.astype(np.float64)
+  want_dz = (want - E64 * (E64 * want).sum(1, keepdims=True)) * rinv[:, None] * np.where(E64 > 0, 1.0, alpha)
+  Ed, nd, rd = dev_t(cd, E), dev_t(cd, neg), dev_t(cd, rinv)
+  got = [cd.ops.triplet_hinge(Ed, B, margin, neg_row=nd, want_dE=True)["dE"].cpu().numpy() for _ in range(3)]
+  assert 0.3 < (h > 0).mean() < 0.9                                                 # active and inactive triplets
+  assert np.all(np.abs(got[0] - want) <= 1e-6 * bound + 1e-7)
+  assert np.array_equal(got[0], got[1]) and np.array_equal(got[0], got[2])
+  dz = []
+  for _ in range(2):
+    ws = torch.full((3 * B * D,), float("nan"), dtype=torch.float32, device=cd.dev)
+    dz16 = torch.empty((3 * B, D), dtype=torch.float16, device=cd.dev)
+    cd.ops.triplet_hinge(Ed, B, margin, neg_row=nd, rinv=rd, leaky_alpha=alpha, dz16=dz16, workspace=ws)
+    assert np.array_equal(ws.view(3 * B, D).cpu().numpy(), got[0])
+    dz.append(dz16.float().cpu().numpy())
+  assert np.array_equal(dz[0], dz[1])
+  live = np.abs(want_dz).sum(1) > 0
+  assert rel_rows(dz[0][live], want_dz[live]).max() < 2e-3                           # fp16 output
+
+
 # ---------------------------------------------------------------- K2-K4 forward
 @pytest.mark.parametrize("dims,rows", [([1500, 5000, 256], 3 * 171), ([64, 128, 256], 3 * 50), ([2048, 2048, 2048, 2048, 256], 3 * 64)])
 def test_tower_forward_embeddings_within_1e3(cd, dims, rows):
