@@ -199,7 +199,7 @@ static int launch_gemm_resb(cdml_ctx* ctx, const void* A, int64_t lda, const voi
   const int grid = static_cast<int>(units < ctx->num_sms ? units : ctx->num_sms);
   kern<<<grid, 128 + 32 * kEpiWarps, L::kTotal, stream>>>(ta, tb, s, epi);
   CDML_CHECK_CUDA(cudaGetLastError());
-  if (trace_sync("gemm_resb", M, N, K, grid, stream)) return -2;
+  if (trace_sync(Epi::kTmaStore ? "gemm_resb[tma]" : "gemm_resb", M, N, K, grid, stream)) return -2;
   return 1;
 }
 

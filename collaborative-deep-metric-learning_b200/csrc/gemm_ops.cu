@@ -63,7 +63,10 @@ static int dispatch_epilogue(cdml_ctx* ctx, const void* A, int64_t lda, const vo
           const char* e = getenv("CDML_TMA_STORE");
           tma_on = (e != nullptr && e[0] == '0') ? 0 : 1;
         }
-        if (tma_on && num_splits <= 1 && resb_applicable(K) && M >= 8 * kBM && (ld_out * 2) % 16 == 0) {
+        // N % 8 == 0 as well: a box that crosses the tensor map's inner bound inside a 16-byte piece was found (B200) to
+        // write zeros past column N-1, into the caller's pitch padding or neighbouring columns
+        // (profiles/r03_gemm_exact_on_parent.log; tests/test_gemm_exact.py checks the padding of every output)
+        if (tma_on && num_splits <= 1 && resb_applicable(K) && M >= 8 * kBM && (ld_out * 2) % 16 == 0 && N % 8 == 0) {
           CUtensorMap om;
           int rc = make_tmap_2d(ctx, &om, out, dtype16, N, M, ld_out, 32, 32, 64);
           if (rc) return rc;

@@ -467,6 +467,13 @@ struct EpiMaskBits {
 // the 64-byte TMA swizzle of a [32 rows x 64 bytes] box -- and one lane hands the box to the TMA engine instead of the warp
 // reading it back and issuing 4 x 32 sixteen-byte global stores: half the shared-memory traffic and a quarter of the LSU
 // instructions of the staged path, full 64-byte row pieces, M / N tails clipped by the tensor map.
+//
+// Slice reuse.  A box is staged after `wait_group.read 1` (every committed box except the newest has left shared memory),
+// which is safe only if the newest box came from the OTHER slice.  Invariant: every tile's last box comes from slice 1.
+// So a tile of n boxes (the ok() chunks are a prefix: cc = 0 .. n-1) stages box cc in slice (cc + n) & 1.  With n even
+// the first box takes slice 0 and `read 1` suffices; with n odd (the last column block when N mod 256 lies in (0,32],
+// (64,96], (128,160] or (192,224]) the first box takes slice 1, where the previous tile's last box may still be read,
+// and waits with `read 0` -- for a box committed before the previous tile's epilogue ended, not for the one just issued.
 template <int BN, int kBf16>
 struct EpiMaskBitsTma {
   static constexpr bool kSplitColumns = true;
@@ -499,6 +506,7 @@ struct EpiMaskBitsTma {
     const int lane = threadIdx.x & 31;
     const int row_base = row - lane;
     auto ok = [&](int cc) { return c0 + cc < c1 && n0 + (c0 + cc) * 32 < s.N; };   // warp-uniform
+    const int boxes = ok(0) + ok(1) + ok(2) + ok(3);
     auto chunk = [&](const uint32_t (&v)[32], int cc) {
       const uint32_t b = st.bits[cc];
       uint32_t pk[16];
@@ -508,8 +516,11 @@ struct EpiMaskBitsTma {
         const float x1 = __uint_as_float(v[2 * j + 1]) * ((b >> (2 * j + 1)) & 1u ? 1.f : alpha);
         pk[j] = pack2<kBf16>(x0, x1);
       }
-      const uint32_t stg = stg0 + (cc & 1) * 2048u;
-      if (lane == 0) bulk_wait_read1();      // the box written to this slice two chunks ago has left shared memory
+      const uint32_t stg = stg0 + ((cc + boxes) & 1) * 2048u;
+      if (lane == 0) {
+        if (cc == 0 && (boxes & 1)) bulk_wait_read0();   // slice 1 may hold the previous tile's last box
+        else bulk_wait_read1();                          // the newest box came from the other slice
+      }
       __syncwarp();
 #pragma unroll
       for (int j = 0; j < 4; ++j)

@@ -157,7 +157,8 @@ def test_tower_forward_embeddings_within_1e3(cd, dims, rows):
 def test_sign_mask_forward_and_mask_bits_data_gradient(cd, t16, R, N, K):
   """The packed sign mask (STORE_16 aux0) is exactly `activation > 0`, bit for bit, and the MASK_BITS data gradient equals
   the MASK_LEAKY one (which reads the 16-bit activation) bit for bit -- on the resident-B kernel (R >= 1024) and the
-  generic one, ragged N, both operand types."""
+  generic one, ragged N, both operand types.  (mask == (H > 0) only outside the band where a positive pre-activation rounds
+  to a 16-bit +0, (0, 2^-25] in fp16; these random inputs do not reach it, test_gemm_exact.py covers it.)"""
   from cdml_b200._lib import EPI_MASK_BITS, EPI_MASK_LEAKY, EPI_STORE_16
   gen = torch.Generator(device=cd.dev)
   gen.manual_seed(R + N)

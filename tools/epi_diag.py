@@ -18,6 +18,7 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--batch", type=int, default=65536)
 ap.add_argument("--reps", type=int, default=5)
 ap.add_argument("--only", default="", help="comma list of sections: scan, mine-structureless, mine-clustered, mine-random-sphere, dgrad")
+ap.add_argument("--dgrad-n", type=int, default=5000, help="output columns of the dgrad section (5000: VNet, 1500: fusion towers)")
 ap.add_argument("--no-warm", action="store_true", help="no untimed warm-up call (ncu captures: one launch per kernel)")
 args = ap.parse_args()
 only = set(x for x in args.only.split(",") if x)
@@ -75,8 +76,8 @@ for regime in ("structureless", "clustered", "random-sphere"):
   mined = float((neg.long() != 3 * torch.arange(B, device=dev) + 2).float().mean().item())
   print("mining %-14s %.3f ms for both scans + prepare/finalize (%.0f TFLOP/s), mined fraction %.3f" % (regime, ms, 2 * flop / ms / 1e9, mined))
 
-# data gradient: dz2 [R,256] x W2 [5000,256]^T -> [R,5000] masked by the sign of h1
-R, N = 3 * B, 5000
+# data gradient: dz2 [R,256] x W2 [N,256]^T -> [R,N] masked by the sign of h1 (N = 5000: VNet's layer 1)
+R, N = 3 * B, args.dgrad_n
 pad = lambda n: (n + 63) // 64 * 64
 dz = (torch.randn((R, D), generator=gen, device=dev) * 0.1).half()
 W = (torch.randn((N, D), generator=gen, device=dev) * 0.1).half()
