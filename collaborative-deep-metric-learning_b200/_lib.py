@@ -48,6 +48,8 @@ _SIGNATURES = {
   "cdml_cast16": (c_int, [_P, _P, c_int64, _P, c_int, _P]),
   "cdml_fill_column16": (c_int, [_P, _P, c_int64, c_int64, c_int64, c_float, c_int, _P]),
   "cdml_mine_semihard": (c_int, [_P, _P, c_int64, c_int, _P, c_int64, _P, c_int64, c_int, c_float, _P, _P, _P]),
+  "cdml_mine_distance_weighted": (c_int, [_P, _P, c_int64, c_int, _P, c_int64, _P, c_int64, c_int, c_float, c_float,
+                                          ctypes.c_uint64, _P, _P, _P, _P]),
   "cdml_mine_last_stats": (c_int, [_P, _P, _P]),
   "cdml_knn_index_build": (c_int, [_P, _P, c_int64, c_int, c_int64, c_int, _P, POINTER(c_void_p)]),
   "cdml_knn_index_destroy": (c_int, [_P]),

@@ -221,6 +221,29 @@ __device__ __forceinline__ float fmax3(float a, float b, float c) {
   return r;
 }
 __device__ __forceinline__ uint32_t umin3(uint32_t a, uint32_t b, uint32_t c) { return __vimin3_u32(a, b, c); }
+__device__ __forceinline__ uint32_t umax3(uint32_t a, uint32_t b, uint32_t c) { return __vimax3_u32(a, b, c); }
+
+__device__ __forceinline__ uint32_t f2key(float f) {  // order-preserving float -> uint32
+  const uint32_t u = __float_as_uint(f);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float key2f(uint32_t k) {
+  return __uint_as_float((k & 0x80000000u) ? (k & 0x7FFFFFFFu) : ~k);
+}
+
+// Philox4x32-10 (Salmon et al., SC'11; pinned in tests to the Random123 known-answer vectors): the four output words of
+// counter (c0, c1, c2, c3) under key (k0, k1).
+__device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
+                                               uint32_t k1) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
+    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
+    c0 = hi1 ^ c1 ^ k0, c1 = lo1, c2 = hi0 ^ c3 ^ k1, c3 = lo0;
+    k0 += 0x9E3779B9u, k1 += 0xBB67AE85u;
+  }
+  return make_uint4(c0, c1, c2, c3);
+}
 
 // ----------------------------------------------------------------------------------------------
 // 16-bit element helpers (dtype 0 = fp16, 1 = bf16)

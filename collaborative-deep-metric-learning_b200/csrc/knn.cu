@@ -27,13 +27,6 @@ constexpr int kKeepCap = 2048;   // survivors of the approximate prune that get 
 constexpr int kMaxGroups = 4096; // sample groups per query (sample <= 131072 rows)
 constexpr int kRefineThreads = 256;
 
-__device__ __forceinline__ uint32_t f2key(float f) {  // order-preserving float -> uint32
-  const uint32_t u = __float_as_uint(f);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float key2f(uint32_t k) {
-  return __uint_as_float((k & 0x80000000u) ? (k & 0x7FFFFFFFu) : ~k);
-}
 __device__ __forceinline__ float neg_inf() { return __int_as_float(0xff800000); }
 __device__ __forceinline__ float pos_inf() { return __int_as_float(0x7f800000); }
 

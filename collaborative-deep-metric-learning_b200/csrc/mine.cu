@@ -224,6 +224,189 @@ struct EpiMine {
   }
 };
 
+// Distance-weighted negative sampling (Wu et al. 2017, "Sampling Matters in Deep Embedding Learning"), the second mining
+// mode.  Same candidates as EpiMine.  With delta = max(2 - 2s, dmin) (dmin = cutoff^2), a candidate is eligible iff
+// delta < dp + margin, and the pick is argmin over eligible candidates of key = ln E - log w(delta), E ~ Exp(1) iid per
+// (anchor, candidate): an exponential race, P(pick j) = w_j / sum w.  log w is the inverse density of squared distances
+// between uniform points of the unit sphere in D dimensions:
+//   log w(delta) = -((D-2)/2) ln delta - ((D-3)/2) ln max(1 - delta/4, kDwOneMinusMin).
+// Draws, per 32-column chunk of a launch (chunk id = 2 * (column / 32) + cand - 1), from Philox4x32-10 with key = seed and
+// counter = (anchor, chunk id, step lo, (step hi << 4) | w); a word x maps to U = ((x >> 9) + 0.5) 2^-23, Exp(1) = -ln U.
+//   w = 0: M = Exp(1) / 32 from word 0 (the chunk's minimum, Exp(32)), K = word 1 >> 27 (its column),
+//   w = 1..8: word t gives X_j for column j = 4 (w - 1) + t;  E_j = M for j = K, M + X_j otherwise.
+// By memorylessness and symmetry the E_j are 32 iid Exp(1), and every E_j >= M.  Common path per chunk: the score range
+// (packed sub + 3-input min/max over t = 2 - s > 0, as EpiMine) bounds delta to [dlo, dhi]; log w is U-shaped (minimum
+// at delta = 4(D-2)/(2D-5)), so L = max(log w(dlo), log w(dhi)) bounds it over the chunk, and ln M - L bounds every key.
+// Only a chunk whose bound beats the anchor's best key draws the other 31 E_j and evaluates the exact keys (re-scan).
+// Result: 64-bit key (f2key(key) << 32 | row) folded with atomicMin -> ties go to the lowest row.
+constexpr float kDwOneMinusMin = 1e-6f;
+constexpr float kDwLnMFloor = -20.5f;   // ln M >= ln(-ln(1 - 2^-24) / 32) = -20.1 for every draw: skips the Philox call
+
+__device__ __forceinline__ float dw_exp1(uint32_t x) {   // accurate log: relative precision of E near 0 matters
+  return -logf((static_cast<float>(x >> 9) + 0.5f) * 0x1p-23f);
+}
+
+template <int BN>
+struct EpiMineDW {
+  static constexpr bool kSplitColumns = true;
+  static constexpr bool kPrefetchNext = false;
+  static constexpr bool kRowConsts = false;
+  static constexpr bool kEarlyRelease = true;
+  static constexpr bool kTmaStore = false;
+  struct State {
+    float dpm;            // dp + margin: eligible iff delta < dpm
+    int ga, gp;
+    uint32_t bkey, brow;  // the anchor's best (key, row) so far, from the global key at tile start
+    uint32_t release_bar;
+  };
+  const float* dp;
+  const int32_t* guid;
+  unsigned long long* best;  // [B] f2key(key) << 32 | row
+  int cand;
+  unsigned long long* stats;
+  float margin, dmin, ha, hb;   // dmin = cutoff^2, ha = (D-2)/2, hb = (D-3)/2
+  uint32_t seed_lo, seed_hi;
+  const int64_t* step;          // device step counter (nullptr: 0), read at every launch so graph replays draw anew
+  __device__ __forceinline__ float logw(float delta) const {
+    return -(ha * __logf(delta) + hb * __logf(fmaxf(fmaf(-0.25f, delta, 1.f), kDwOneMinusMin)));
+  }
+  __device__ __forceinline__ void pre(State& st, int row, int /*n0*/, const GemmShape& s, int, int, uint32_t) const {
+    const bool row_ok = row < s.M;
+    st.dpm = row_ok ? __ldg(dp + row) + margin : -__int_as_float(0x7f800000);   // rows beyond M: nothing eligible
+    st.ga = row_ok ? __ldg(guid + 3 * row) : 0;
+    st.gp = row_ok ? __ldg(guid + 3 * row + 1) : 0;
+    const unsigned long long key = row_ok ? best[row] : ~0ull;
+    st.bkey = static_cast<uint32_t>(key >> 32), st.brow = static_cast<uint32_t>(key);
+    st.release_bar = 0u;
+  }
+  __device__ __forceinline__ void cols(int n0, const GemmShape& s, int c0, int /*c1*/, uint32_t stg) const {
+    static_assert(BN == 256, "a warp owns 4 chunks (128 columns) of the tile");
+    col_cache_fill(stg, n0, c0, [&](int col) { return static_cast<uint32_t>(col < s.N ? __ldg(guid + 3 * col + cand) : -1); });
+  }
+  __device__ __forceinline__ void block_begin(uint32_t epi_smem) const { col_cache_reset(epi_smem); }
+  __device__ __forceinline__ void block_end(uint32_t) const {}
+  __device__ __forceinline__ void run(uint32_t taddr, int row, int n0, int /*split*/, const GemmShape& s, int c0,
+                                      int c1, uint32_t stg, State& st) const {
+    const int lane = threadIdx.x & 31;
+    const float inf = __int_as_float(0x7f800000);
+    const float dpm = st.dpm;
+    const int ga = st.ga, gp = st.gp;
+    uint32_t bkey = st.bkey, brow = st.brow;
+    float bf = key2f(bkey);
+    if (!(bf == bf)) bf = inf;   // empty key reads as NaN
+    bool found = false;
+    const uint64_t stp = step != nullptr ? static_cast<uint64_t>(__ldg(step)) : 0ull;
+    const uint32_t ctr2 = static_cast<uint32_t>(stp), ctr3 = static_cast<uint32_t>(stp >> 32) << 4;
+    uint32_t va[32], vb[32];
+    // exact key of column j's score sc given its draw word x (unused for j == K); +inf when not eligible
+    auto key_of = [&](float sc, int j, uint32_t x, float M, uint32_t K, float dpm_, int g, int ga_, int gp_) {
+      const float delta = fmaxf(fmaf(-2.f, sc, 2.f), dmin);
+      const float E = static_cast<uint32_t>(j) == K ? M : M + dw_exp1(x);
+      const bool pass = delta < dpm_ && g != ga_ && g != gp_ && g >= 0;
+      return pass ? f2key(__logf(E) - logw(delta)) : 0xffffffffu;
+    };
+    auto chunk = [&](const uint32_t (&v)[32], int cc) {
+      const int nb = n0 + (c0 + cc) * 32;
+      const uint32_t cid = 2u * static_cast<uint32_t>(nb >> 5) + static_cast<uint32_t>(cand - 1);
+      // t = 2 - s > 0 for every score, so the raw bits order like the values: min/max of t = the chunk's score range
+      uint32_t u0 = 0xffffffffu, u1 = 0xffffffffu, w0 = 0u, w1 = 0u;
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const float2 lo = sub2(2.f, 2.f, __uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]));
+        const float2 hi = sub2(2.f, 2.f, __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
+        u0 = umin3(u0, __float_as_uint(lo.x), __float_as_uint(lo.y));
+        u1 = umin3(u1, __float_as_uint(hi.x), __float_as_uint(hi.y));
+        w0 = umax3(w0, __float_as_uint(lo.x), __float_as_uint(lo.y));
+        w1 = umax3(w1, __float_as_uint(hi.x), __float_as_uint(hi.y));
+      }
+      const float dlo = fmaxf(fmaf(2.f, __uint_as_float(min(u0, u1)), -2.f), dmin);
+      const float dhi = fminf(fmaxf(fmaf(2.f, __uint_as_float(max(w0, w1)), -2.f), dmin), dpm);
+      float L = fmaxf(logw(dlo), logw(dhi));
+      L += 1e-3f + 1e-4f * fabsf(L);   // covers the rounding of t, delta and the approximate logs
+      float M = 0.f;
+      uint32_t K = 0u;
+      bool hit = dlo < dpm && kDwLnMFloor - L < bf;
+      if (hit) {
+        const uint4 x = philox4x32_10(static_cast<uint32_t>(row), cid, ctr2, ctr3, seed_lo, seed_hi);
+        M = dw_exp1(x.x) * (1.f / 32.f), K = x.y >> 27;
+        hit = __logf(M) - L < bf;
+      }
+      unsigned int hits = __ballot_sync(0xffffffffu, hit);
+      if (hits == 0u) return;
+      if (lane == 0) atomicAdd(stats, static_cast<unsigned long long>(__popc(hits)));
+      if (__popc(hits) >= kMassHits) {
+        // many rows at once (first visits, while the bounds are loose): every hitting thread scans its own 32 columns
+        if (hit) {
+          uint32_t kbest = 0xffffffffu;
+          int cbest = -1;
+#pragma unroll
+          for (int w = 0; w < 8; ++w) {
+            const uint4 x = philox4x32_10(static_cast<uint32_t>(row), cid, ctr2, ctr3 | (w + 1), seed_lo, seed_hi);
+            const uint32_t xs[4] = {x.x, x.y, x.z, x.w};
+#pragma unroll
+            for (int t = 0; t < 4; ++t) {
+              const int j = 4 * w + t;
+              int g;
+              asm volatile("ld.shared.b32 %0, [%1];" : "=r"(g) : "r"(stg + kColCacheOff + 128 * cc + 4 * j) : "memory");
+              const uint32_t k = key_of(__uint_as_float(v[j]), j, xs[t], M, K, dpm, g, ga, gp);
+              if (k < kbest) kbest = k, cbest = j;
+            }
+          }
+          const uint32_t r = static_cast<uint32_t>(3 * (nb + cbest) + cand);
+          if (cbest >= 0 && (kbest < bkey || (kbest == bkey && r < brow))) bkey = kbest, brow = r, bf = key2f(kbest), found = true;
+        }
+        __syncwarp();
+      } else {
+        int g_lane;   // candidate guid of column nb + lane (column cache)
+        asm volatile("ld.shared.b32 %0, [%1];" : "=r"(g_lane) : "r"(stg + kColCacheOff + 128 * cc + 4 * lane) : "memory");
+        do {   // one hitting row at a time: lane j evaluates column j (its draw is word j % 4 of call 1 + j / 4)
+          const int src = __ffs(hits) - 1;
+          hits &= hits - 1u;
+          __syncwarp();
+          if (lane == src) {
+#pragma unroll
+            for (int j = 0; j < 8; ++j) sts128(stg + 16 * j, v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+          }
+          __syncwarp();
+          float sc;
+          asm volatile("ld.shared.f32 %0, [%1];" : "=f"(sc) : "r"(stg + 4 * lane) : "memory");
+          const int row_s = __shfl_sync(0xffffffffu, row, src);
+          const float M_s = __shfl_sync(0xffffffffu, M, src), dpm_s = __shfl_sync(0xffffffffu, dpm, src);
+          const uint32_t K_s = __shfl_sync(0xffffffffu, K, src);
+          const int ga_s = __shfl_sync(0xffffffffu, ga, src), gp_s = __shfl_sync(0xffffffffu, gp, src);
+          const uint4 x = philox4x32_10(static_cast<uint32_t>(row_s), cid, ctr2, ctr3 | (1 + (lane >> 2)), seed_lo, seed_hi);
+          const int t = lane & 3;
+          const uint32_t xw = t == 0 ? x.x : t == 1 ? x.y : t == 2 ? x.z : x.w;
+          const uint32_t k = key_of(sc, lane, xw, M_s, K_s, dpm_s, g_lane, ga_s, gp_s);
+          const uint32_t kmin = __reduce_min_sync(0xffffffffu, k);
+          if (kmin != 0xffffffffu) {   // warp-uniform
+            const int col = __ffs(__ballot_sync(0xffffffffu, k == kmin)) - 1;
+            const uint32_t r = static_cast<uint32_t>(3 * (nb + col) + cand);
+            if (lane == src && (kmin < bkey || (kmin == bkey && r < brow))) bkey = kmin, brow = r, bf = key2f(kmin), found = true;
+          }
+        } while (hits != 0u);
+      }
+    };
+    auto ok = [&](int cc) { return c0 + cc < c1 && n0 + (c0 + cc) * 32 < s.N; };   // warp-uniform
+    tmem_ld_32x32(taddr + c0 * 32, va);
+#pragma unroll
+    for (int cc = 0; cc < 4; cc += 2) {
+      tmem_ld_wait();
+      if (ok(cc + 1)) tmem_ld_32x32(taddr + (c0 + cc + 1) * 32, vb);
+      if (ok(cc)) chunk(va, cc);
+      tmem_ld_wait();
+      if (cc + 2 < 4 && ok(cc + 2)) tmem_ld_32x32(taddr + (c0 + cc + 2) * 32, va);
+      if (cc + 2 >= 4 && st.release_bar != 0u) {   // every TMEM read of this warp has landed: release the buffer now
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(st.release_bar);
+      }
+      if (ok(cc + 1)) chunk(vb, cc + 1);
+    }
+    if (found) atomicMin(best + row, (static_cast<unsigned long long>(bkey) << 32) | brow);
+  }
+};
+
 __global__ void mine_prepare_kernel(const float* __restrict__ E, int64_t ld, int D, const int64_t* __restrict__ guid64,
                                     int64_t B, float* __restrict__ dp, int32_t* __restrict__ guid32,
                                     unsigned long long* __restrict__ best, unsigned long long* __restrict__ stats) {
@@ -308,6 +491,43 @@ extern "C" int cdml_mine_semihard(cdml_ctx* ctx, const void* E16, int64_t ld16, 
     } else if (resb_applicable(D) && B >= 8 * kBM && epi_warps() == 16)
       rc = launch_gemm_resb<EpiMine<kBN, 1>, 16>(ctx, e16, 3 * ld16, e16 + cand * ld16, 3 * ld16, B, B, D, dtype16, epi, st);
     else if (resb_applicable(D) && B >= 8 * kBM)
+      rc = launch_gemm_resb(ctx, e16, 3 * ld16, e16 + cand * ld16, 3 * ld16, B, B, D, dtype16, epi, st);
+    else
+      rc = launch_gemm<0, 0>(ctx, e16, 3 * ld16, e16 + cand * ld16, 3 * ld16, B, B, D, dtype16, 1, epi, st);
+  }
+  if (rc >= 0) {
+    mine_finalize_kernel<<<grid, 256, 0, st>>>(E32, ld32, D, best, B, neg_row, d_an, stats);
+    rc = cudaGetLastError() == cudaSuccess ? 0 : -2;
+  }
+  return rc < 0 ? rc : 0;
+}
+
+extern "C" int cdml_mine_distance_weighted(cdml_ctx* ctx, const void* E16, int64_t ld16, int dtype16, const float* E32,
+                                           int64_t ld32, const int64_t* guid, int64_t B, int D, float margin, float cutoff,
+                                           uint64_t seed, const int64_t* step, int32_t* neg_row, float* d_an,
+                                           void* stream) {
+  CDML_REQUIRE(ctx && E16 && E32 && guid && neg_row, "cdml_mine_distance_weighted: NULL argument");
+  CDML_REQUIRE(B > 0 && 3 * B < (1ll << 31) && D >= 8 && D % 8 == 0 && ld16 >= D && ld32 >= D,
+               "cdml_mine_distance_weighted: bad geometry B=%lld D=%d", (long long)B, D);
+  CDML_REQUIRE(cutoff > 0.f && cutoff < 2.f && margin == margin, "cdml_mine_distance_weighted: cutoff %g not in (0, 2)",
+               (double)cutoff);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const size_t bytes = static_cast<size_t>(B) * (8 + 4 + 12) + 64;   // as cdml_mine_semihard
+  uint8_t* ws = static_cast<uint8_t*>(ctx_scratch(ctx, bytes));
+  if (ws == nullptr) return -2;
+  if (ctx->mine_stats == nullptr) CDML_CHECK_CUDA(cudaMalloc(&ctx->mine_stats, 2 * sizeof(unsigned long long)));
+  unsigned long long* stats = ctx->mine_stats;
+  unsigned long long* best = reinterpret_cast<unsigned long long*>(ws);
+  float* dp = reinterpret_cast<float*>(best + B);
+  int32_t* guid32 = reinterpret_cast<int32_t*>(dp + B);
+  const int grid = static_cast<int>(std::min<int64_t>((B + 7) / 8, ctx->num_sms * 8));
+  mine_prepare_kernel<<<grid, 256, 0, st>>>(E32, ld32, D, guid, B, dp, guid32, best, stats);
+  int rc = 0;
+  const uint16_t* e16 = static_cast<const uint16_t*>(E16);
+  for (int cand = 1; cand <= 2 && rc >= 0; ++cand) {
+    EpiMineDW<kBN> epi{dp, guid32, best, cand, stats, margin, cutoff * cutoff, 0.5f * (D - 2), 0.5f * (D - 3),
+                       static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32), step};
+    if (resb_applicable(D) && B >= 8 * kBM)
       rc = launch_gemm_resb(ctx, e16, 3 * ld16, e16 + cand * ld16, 3 * ld16, B, B, D, dtype16, epi, st);
     else
       rc = launch_gemm<0, 0>(ctx, e16, 3 * ld16, e16 + cand * ld16, 3 * ld16, B, B, D, dtype16, 1, epi, st);

@@ -94,6 +94,9 @@ class TowerEngine:
     self.gb = [self._view(self.g, 2 * l + 1) for l in range(self.L)]
     self.W16 = [torch.zeros(self.shapes[l], dtype=self.t16, device=dev) for l in range(self.L)]
     self.step_counter = torch.zeros(1, dtype=torch.int64, device=dev)
+    # distance-weighted mining (mine="distance_weighted"): distance cutoff and the seed of its draws; the draws of a step
+    # are also keyed by step_counter, which the kernel reads from device memory (a replayed graph draws afresh)
+    self.dw_cutoff, self.dw_seed = 0.5, int(seed)
     self.scalars = torch.zeros(4, dtype=torch.float32, device=dev)
     self.norms = torch.zeros((2 * self.L, 2), dtype=torch.float32, device=dev)       # per variable: {sum g_eff^2, sum w^2}
     self.opt_ws = torch.empty((ops.opt_workspace_floats(),), dtype=torch.float32, device=dev)
@@ -287,9 +290,7 @@ class TowerEngine:
       if e16 is None:
         e16 = self._ws[("e16", R)] = torch.empty((R, D), dtype=self.t16, device=self.device)
     buf = self.forward_rows(x16, R, train=True, want_e16=e16)
-    neg_row = None
-    if mine:
-      neg_row, _ = ops.mine_semihard(e16, buf["e"], guid, B, self.margin, want_dist=False)
+    neg_row = self._mine_negatives(e16, buf["e"], guid, B, mine) if mine else None
     dz = buf["dz"]
     # loss + backward through the output L2-norm and last leaky (gradients of the SUM of hinges; 1/B goes into Adam)
     ops.triplet_hinge(buf["e"], B, self.margin, neg_row=neg_row, grad_scale=1.0, rinv=buf["rinv"],
@@ -297,6 +298,16 @@ class TowerEngine:
     self.backward_rows(x16, R, buf, input_ones)
     self.apply_gradients(B)
     return buf["loss"]["stats"]
+
+  def _mine_negatives(self, e16, e, guid, B, mine):
+    """In-batch negatives of a training step.  mine: True or "semihard" -> semi-hard mining; "distance_weighted" ->
+    distance-weighted sampling with (dw_cutoff, dw_seed) at the current step_counter."""
+    if mine is True or mine == "semihard":
+      return ops.mine_semihard(e16, e, guid, B, self.margin, want_dist=False)[0]
+    if mine == "distance_weighted":
+      return ops.mine_distance_weighted(e16, e, guid, B, self.margin, self.dw_cutoff, self.dw_seed, self.step_counter,
+                                        want_dist=False)[0]
+    raise ValueError("mine must be False, True, 'semihard' or 'distance_weighted' (got %r)" % (mine,))
 
   def backward_rows(self, x16, R, buf, input_ones=False):
     dz = buf["dz"]

@@ -226,9 +226,7 @@ class GraphEngine(TowerEngine):
       if e16 is None:
         e16 = self._ws[("e16", R)] = torch.empty((R, self.widths[-1]), dtype=self.t16, device=self.device)
     buf = self.forward_rows(xsegs, R, train=True, want_e16=e16)
-    neg_row = None
-    if mine:
-      neg_row, _ = ops.mine_semihard(e16, buf["e"], guid, B, self.margin, want_dist=False)
+    neg_row = self._mine_negatives(e16, buf["e"], guid, B, mine) if mine else None
     # loss + backward through the output L2-norm (and the last leaky when the output fc is fused)
     ops.triplet_hinge(buf["e"], B, self.margin, neg_row=neg_row, grad_scale=self.loss_scale, rinv=buf["rinv"],
                       leaky_alpha=self.alpha if self.fused_out is not None else 1.0, dz16=buf["dzo"],

@@ -306,8 +306,27 @@ def mine_semihard(E16, E32, guid, B, margin, want_dist=True):
   return neg_row, d_an
 
 
+def mine_distance_weighted(E16, E32, guid, B, margin, cutoff=0.5, seed=0, step=None, want_dist=True):
+  """Distance-weighted negative sampling (Wu et al. 2017): neg_row [B] int32 sampled among the candidates with
+  max(d, cutoff^2) < |a-p|^2 + margin with probability ~ 1/q(d), q the density of distances on the unit sphere; d_an the
+  exact fp32 distance of the pick (want_dist).  step: a one-element int64 device tensor read by the kernel (the engine's
+  step counter, so that graph replays draw afresh), or None for step 0."""
+  D = E32.shape[1]
+  if step is not None and (step.dtype != torch.int64 or step.device != E32.device or step.numel() < 1):
+    raise ValueError("mine_distance_weighted: step must be an int64 tensor on %s" % E32.device)
+  neg_row = torch.empty((B,), dtype=torch.int32, device=E32.device)
+  d_an = torch.empty((B,), dtype=torch.float32, device=E32.device) if want_dist else None
+  guid = guid.to(torch.int64).contiguous()
+  _count(4)
+  check(_lib.load().cdml_mine_distance_weighted(_ctx(E32), ptr(E16), E16.stride(0), dtype16_of(E16), ptr(E32),
+                                                E32.stride(0), ptr(guid), B, D, float(margin), float(cutoff),
+                                                int(seed) & 0xFFFFFFFFFFFFFFFF, ptr(step), ptr(neg_row), ptr(d_an),
+                                                stream_ptr()))
+  return neg_row, d_an
+
+
 def mine_stats(ref):
-  """Diagnostics of the last mine_semihard on ref's device: {"rescans": re-scanned (anchor, 32-candidate chunk) pairs,
+  """Diagnostics of the last mine_semihard or mine_distance_weighted on ref's device: {"rescans": re-scanned (anchor, 32-candidate chunk) pairs,
   "mined": anchors that received a mined negative}.  Synchronises the current stream."""
   out = (ctypes.c_int64 * 2)()
   check(_lib.load().cdml_mine_last_stats(_ctx(ref), out, stream_ptr()))

@@ -34,6 +34,9 @@ if "train_dir" not in FLAGS:
   flags.DEFINE_integer("num_epochs", 8, "passes over each *.train file (train.py:359)")
   flags.DEFINE_integer("batch_size", 1024, "triplets per step (train.py:360)")
   flags.DEFINE_boolean("mine_semihard", False, "in-batch semi-hard negative mining (SURVEY 8a row M)")
+  flags.DEFINE_boolean("mine_distance_weighted", False, "in-batch distance-weighted negative sampling (Wu et al. 2017); "
+                       "not together with --mine_semihard")
+  flags.DEFINE_float("dw_cutoff", 0.5, "distance cutoff of --mine_distance_weighted: closer candidates weigh as this distance")
   flags.DEFINE_boolean("device_reader", False, "sample the index triplets on the GPU (cdml_sample_triplets; SURVEY 8f row 3)")
   flags.DEFINE_string("compute_dtype", "fp16", "tensor-core operand type: fp16 | bf16 (fp32 accumulate)")
 
@@ -200,7 +203,12 @@ class Trainer():
   def __init__(self, pipe, num_epochs, batch_size, model, loss_fn, learning_rate, margin,
                checkpoint_dir, optimizer_class, config, eval_cowatches, test_cowatches,
                check_stop_epoch, best_eval_dist=1.0, eval_per_epoch=100, require_improve_num=10,
-               mine_semihard=False, dtype16="fp16", process_group=None, max_steps=None):
+               mine_semihard=False, dtype16="fp16", process_group=None, max_steps=None, mine_mode=None, dw_cutoff=0.5):
+    """mine_mode: None (mine_semihard decides), "semihard" or "distance_weighted" (with dw_cutoff)."""
+    if mine_mode not in (None, "semihard", "distance_weighted"):
+      raise ValueError("mine_mode must be None, 'semihard' or 'distance_weighted' (got %r)" % (mine_mode,))
+    if mine_mode == "distance_weighted" and mine_semihard:
+      raise ValueError("mine_semihard and mine_mode='distance_weighted' exclude each other")
     self.pipe, self.num_epochs, self.batch_size = pipe, num_epochs, batch_size
     self.model, self.loss_fn = model, loss_fn
     self.learning_rate, self.margin = learning_rate, margin
@@ -215,6 +223,8 @@ class Trainer():
     self.evaluater = Evaluation(inputs.FEATURES, eval_cowatches)
     self.tester = Evaluation(inputs.FEATURES, test_cowatches)
     self.mine_semihard, self.dtype16, self.pg, self.max_steps = mine_semihard, dtype16, process_group, max_steps
+    self.mine = mine_mode or bool(mine_semihard)      # the engines' `mine` argument
+    self.dw_cutoff = float(dw_cutoff)
     self.is_master = process_group is None or torch.distributed.get_rank(process_group) == 0
     self.history = []
 
@@ -260,6 +270,7 @@ class Trainer():
     F = feature_size() if not isinstance(inputs.FEATURES, np.ndarray) else inputs.FEATURES.shape[1]
     graph = self._build_model(models.placeholder(F, name="input_batch"))
     engine = graph.engine
+    engine.dw_cutoff = self.dw_cutoff
     predictor = Prediction(sess=engine)
     fused = hasattr(self.pipe, "get_batch_indices")
     table16 = engine.prepare_table(self.pipe.device_features()) if fused else None
@@ -267,7 +278,7 @@ class Trainer():
     # (every rank captures and replays the same number of times: the reader serves whole rounds of `world` batches);
     # CDML_DDP_GRAPH=0 keeps data-parallel steps eager
     use_graph = fused and (engine.world == 1 or os.environ.get("CDML_DDP_GRAPH", "1") != "0")
-    replay = engine.capture_step(table16, self.batch_size, mine=self.mine_semihard) if use_graph else None
+    replay = engine.capture_step(table16, self.batch_size, mine=self.mine) if use_graph else None
 
     world = engine.world
     global_step_np = 0
@@ -300,7 +311,7 @@ class Trainer():
 
         batch_start_time = time.time()
         if fused:
-          stats = replay(batch) if replay is not None else engine.train_step_indices(table16, batch, mine=self.mine_semihard)
+          stats = replay(batch) if replay is not None else engine.train_step_indices(table16, batch, mine=self.mine)
         else:
           if batch.shape[1:] != (3, F):
             continue
@@ -333,6 +344,8 @@ class Trainer():
 
 
 def main(args):
+  if FLAGS.mine_semihard and FLAGS.mine_distance_weighted:
+    raise app.UsageError("--mine_semihard and --mine_distance_weighted exclude each other")
   try:
     pg = None
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
@@ -355,7 +368,8 @@ def main(args):
                       optimizer_class=optimizer_class, config=None, eval_cowatches=eval_cowatches,
                       test_cowatches=test_cowatches, check_stop_epoch=3, best_eval_dist=1.0, eval_per_epoch=100,
                       require_improve_num=40, mine_semihard=FLAGS.mine_semihard, dtype16=FLAGS.compute_dtype,
-                      process_group=pg)
+                      process_group=pg, mine_mode="distance_weighted" if FLAGS.mine_distance_weighted else None,
+                      dw_cutoff=FLAGS.dw_cutoff)
     trainer.run()
   except Exception:
     logging.error(traceback.format_exc())

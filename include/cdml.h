@@ -150,7 +150,16 @@ int cdml_fill_column16(cdml_ctx* ctx, void* X16, int64_t rows, int64_t ld, int64
 int cdml_mine_semihard(cdml_ctx* ctx, const void* E16, int64_t ld16, int dtype16, const float* E32, int64_t ld32,
                        const int64_t* guid, int64_t B, int D, float margin, int32_t* neg_row, float* d_an,
                        void* stream);
-/* Diagnostics of the last cdml_mine_semihard on this context (synchronises `stream`): out2[0] = (anchor, 32-candidate
+/* Distance-weighted negative sampling (Wu et al. 2017), the second mining mode: the same candidates and arguments as
+ * cdml_mine_semihard, but the negative is SAMPLED among the candidates with max(d, cutoff^2) < dp + margin, with
+ * probability proportional to the inverse density of squared distances on the unit sphere in D dimensions (the exact
+ * definition and draw layout are stated in csrc/mine.cu and oracle/mine_dw_oracle.py).  Draws are keyed by (seed, *step,
+ * anchor, chunk); step is a device pointer to an int64 read by the kernel (NULL: step 0), so a replayed CUDA graph draws
+ * afresh at every step.  No eligible candidate: row 3i+2. */
+int cdml_mine_distance_weighted(cdml_ctx* ctx, const void* E16, int64_t ld16, int dtype16, const float* E32,
+                                int64_t ld32, const int64_t* guid, int64_t B, int D, float margin, float cutoff,
+                                uint64_t seed, const int64_t* step, int32_t* neg_row, float* d_an, void* stream);
+/* Diagnostics of the last cdml_mine_semihard or cdml_mine_distance_weighted on this context (synchronises `stream`): out2[0] = (anchor, 32-candidate
  * chunk) pairs the selection epilogue had to re-scan, out2[1] = anchors that received a mined negative. */
 int cdml_mine_last_stats(cdml_ctx* ctx, int64_t* out2, void* stream);
 

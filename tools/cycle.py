@@ -33,6 +33,8 @@ ap.add_argument("--lr", type=float, default=1e-4, help="Adam base learning rate 
 ap.add_argument("--no-desim", action="store_true", help="skip the raw-feature KNN + de-similarity stage")
 ap.add_argument("--feat-k", type=int, default=26, help="desim_nearest_num (faiss_knn.py:46)")
 ap.add_argument("--mine", action="store_true", help="in-batch semi-hard mining (default: the reference's random negatives)")
+ap.add_argument("--mine-dw", action="store_true", help="in-batch distance-weighted negative sampling (not with --mine)")
+ap.add_argument("--dw-cutoff", type=float, default=0.5, help="distance cutoff of --mine-dw")
 ap.add_argument("--centre-weight", type=float, default=1.0, help="weight of the cluster centre in a feature row (row = signal * centre + "
                 "noise_weight * U[0,1)); 1.0 / 0.25 = the well-separated default, 0.3 / 1.0 = clusters the tower has to learn")
 ap.add_argument("--noise-weight", type=float, default=0.25)
@@ -81,7 +83,11 @@ tick("build_feature_table_s", t0)
 # ---- stage 1: one training epoch over `triplets` cowatch pairs (anchor/positive from the same cluster, random negative)
 t0 = time.time()
 steps = max(1, args.triplets // B)
-replay = eng.capture_step(table16, B, mine=args.mine)
+if args.mine and args.mine_dw:
+  raise SystemExit("--mine and --mine-dw exclude each other")
+mine = "distance_weighted" if args.mine_dw else args.mine
+eng.dw_cutoff = args.dw_cutoff
+replay = eng.capture_step(table16, B, mine=mine)
 order = torch.argsort(cluster)
 start = torch.searchsorted(cluster[order], torch.arange(NC + 1, device=dev))
 losses = []
@@ -220,7 +226,9 @@ if rank == 0:
                   "eval_cowatch_vs_random_pair_dist_before": eval_before, "eval_cowatch_vs_random_pair_dist_after": eval_after,
                   "features": {"signal": args.centre_weight, "noise": args.noise_weight, "clusters": NC, "lr": args.lr},
                   "top5_same_cluster": same_cluster, "self_is_first_neighbour": self_first,
-                  "knn_fallback_queries_last_block": stats["fallback_queries"], "mining": bool(args.mine), "desim": desim_info,
+                  "knn_fallback_queries_last_block": stats["fallback_queries"], "mining": bool(mine),
+                  "mining_mode": "distance_weighted" if args.mine_dw else "semihard" if args.mine else None,
+                  "dw_cutoff": args.dw_cutoff if args.mine_dw else None, "desim": desim_info,
                   "write_rows_per_rank": R, "write_rows_per_s": R / t["write_s"] if R else None, "out_dir": out_dir}))
 if world > 1:
   torch.distributed.barrier()
