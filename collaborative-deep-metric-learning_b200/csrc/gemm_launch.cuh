@@ -48,16 +48,6 @@ inline int pick_splits(int num_sms, int tiles, int num_kb) {
   return best;
 }
 
-// CDML_2CTA=0 disables the CTA-pair kernel (A/B measurement aid); it is used for tiles of >= 8 k-blocks.
-inline bool two_cta_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("CDML_2CTA");
-    on = (e != nullptr && e[0] == '0') ? 0 : 1;
-  }
-  return on == 1;
-}
-
 template <int AMN, int BMN, class Epi>
 static int launch_gemm2(cdml_ctx* ctx, const void* A, int64_t lda, const void* B, int64_t ldb, int64_t M, int64_t N,
                         int64_t K, int dtype16, int num_splits, const Epi& epi, cudaStream_t stream) {
@@ -107,8 +97,9 @@ template <int AMN, int BMN, class Epi>
 static int launch_gemm(cdml_ctx* ctx, const void* A, int64_t lda, const void* B, int64_t ldb, int64_t M, int64_t N,
                        int64_t K, int dtype16, int num_splits, const Epi& epi, cudaStream_t stream) {
   {
+    // tiles of >= 8 k-blocks run on the CTA-pair kernel
     const int64_t kb_per = ((K + kBK - 1) / kBK + max(num_splits, 1) - 1) / max(num_splits, 1);
-    if (two_cta_enabled() && M >= 2 * kBM && kb_per >= 8)
+    if (M >= 2 * kBM && kb_per >= 8)
       return launch_gemm2<AMN, BMN>(ctx, A, lda, B, ldb, M, N, K, dtype16, num_splits, epi, stream);
   }
   using L = GemmSmem<kBN, kStages>;
@@ -150,16 +141,12 @@ static int launch_gemm(cdml_ctx* ctx, const void* A, int64_t lda, const void* B,
 
 // Resident-B launch (K <= 256, both operands K-major).  Chooses the row-tile chunking so that units fill whole waves.
 constexpr int kResBStages = 4;  // 6 stages (224 KB) leave no L1 for the epilogue's global loads and measured slower
-inline bool resb_applicable(int64_t K) {
-  static int off = -1;   // CDML_NO_RESB=1 forces the generic kernel (A/B measurement aid)
-  if (off < 0) off = getenv("CDML_NO_RESB") != nullptr ? 1 : 0;
-  return off == 0 && K <= 4 * kBK;
-}
+inline bool resb_applicable(int64_t K) { return K <= 4 * kBK; }
 
-template <class Epi, int kEpiWarps = 8>
+template <class Epi>
 static int launch_gemm_resb(cdml_ctx* ctx, const void* A, int64_t lda, const void* B, int64_t ldb, int64_t M, int64_t N,
                             int64_t K, int dtype16, const Epi& epi, cudaStream_t stream, int n_fastest = 0) {
-  using L = ResBSmem<kBN, kResBStages, kEpiWarps, Epi::kRowConsts, Epi::kTmaStore ? 2 : 1>;
+  using L = ResBSmem<kBN, kResBStages, Epi::kTmaStore ? 2 : 1>;
   static_assert(L::kTotal <= 232448, "resident-B kernel: shared memory over the 227 KB limit");
   CUtensorMap ta, tb;
   int rc = make_tmap_2d(ctx, &ta, A, dtype16, K, M, lda, kBK, kBM);
@@ -189,7 +176,7 @@ static int launch_gemm_resb(cdml_ctx* ctx, const void* A, int64_t lda, const voi
   s.tiles_per_chunk = (s.m_tiles + best - 1) / best;
   s.n_fastest = n_fastest;
   s.idesc = make_idesc_f16(dtype16 == CDML_BF16 ? 1 : 0, 0, 0, kBM, kBN);
-  auto kern = gemm_resb_tcgen05_kernel<kBN, kResBStages, Epi, kEpiWarps>;
+  auto kern = gemm_resb_tcgen05_kernel<kBN, kResBStages, Epi>;
   static bool attr_set = false;
   if (!attr_set) {
     CDML_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
@@ -197,7 +184,7 @@ static int launch_gemm_resb(cdml_ctx* ctx, const void* A, int64_t lda, const voi
   }
   const long units = static_cast<long>(s.n_tiles) * s.m_chunks;
   const int grid = static_cast<int>(units < ctx->num_sms ? units : ctx->num_sms);
-  kern<<<grid, 128 + 32 * kEpiWarps, L::kTotal, stream>>>(ta, tb, s, epi);
+  kern<<<grid, kGemmThreads, L::kTotal, stream>>>(ta, tb, s, epi);
   CDML_CHECK_CUDA(cudaGetLastError());
   if (trace_sync(Epi::kTmaStore ? "gemm_resb[tma]" : "gemm_resb", M, N, K, grid, stream)) return -2;
   return 1;

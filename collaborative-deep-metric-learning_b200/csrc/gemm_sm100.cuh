@@ -154,7 +154,6 @@ struct EpiStoreF32 {
   struct State {};
   __device__ __forceinline__ void pre(State&, int, int, const GemmShape&, int, int, uint32_t) const {}
   static constexpr bool kPrefetchNext = false;
-  static constexpr bool kRowConsts = false;
   static constexpr bool kEarlyRelease = false;
   static constexpr bool kTmaStore = false;
   __device__ __forceinline__ void cols(int, const GemmShape&, int, int, uint32_t) const {}
@@ -202,7 +201,6 @@ struct EpiStore16 {
   struct State {};
   __device__ __forceinline__ void pre(State&, int, int, const GemmShape&, int, int, uint32_t) const {}
   static constexpr bool kPrefetchNext = false;
-  static constexpr bool kRowConsts = false;
   static constexpr bool kEarlyRelease = false;
   static constexpr bool kTmaStore = false;
   __device__ __forceinline__ void cols(int, const GemmShape&, int, int, uint32_t) const {}
@@ -251,7 +249,6 @@ struct EpiL2Norm {
   struct State {};
   __device__ __forceinline__ void pre(State&, int, int, const GemmShape&, int, int, uint32_t) const {}
   static constexpr bool kPrefetchNext = false;
-  static constexpr bool kRowConsts = false;
   static constexpr bool kEarlyRelease = false;
   static constexpr bool kTmaStore = false;
   __device__ __forceinline__ void cols(int, const GemmShape&, int, int, uint32_t) const {}
@@ -316,7 +313,6 @@ struct EpiMaskLeaky {
     uint4 raw[4][4];   // the four 32x32 mask chunks of this warp's half-tile, in the coalesced fetch layout
   };
   static constexpr bool kPrefetchNext = false;
-  static constexpr bool kRowConsts = false;
   static constexpr bool kEarlyRelease = false;
   static constexpr bool kTmaStore = false;
   __device__ __forceinline__ void cols(int, const GemmShape&, int, int, uint32_t) const {}
@@ -414,7 +410,6 @@ struct EpiMaskBits {
     uint32_t bits[4];
   };
   static constexpr bool kPrefetchNext = true;
-  static constexpr bool kRowConsts = false;
   static constexpr bool kEarlyRelease = false;
   static constexpr bool kTmaStore = false;
   __device__ __forceinline__ void cols(int, const GemmShape&, int, int, uint32_t) const {}
@@ -482,7 +477,6 @@ struct EpiMaskBitsTma {
     uint32_t release_bar;   // the accumulator buffer's "empty" barrier (kEarlyRelease)
   };
   static constexpr bool kPrefetchNext = true;
-  static constexpr bool kRowConsts = false;
   static constexpr bool kEarlyRelease = true;
   static constexpr bool kTmaStore = true;    // two 2 KB staging slices per warp: a box is written while the previous one drains
   __device__ __forceinline__ void cols(int, const GemmShape&, int, int, uint32_t) const {}
@@ -559,7 +553,6 @@ struct EpiNull {
   struct State {};
   __device__ __forceinline__ void pre(State&, int, int, const GemmShape&, int, int, uint32_t) const {}
   static constexpr bool kPrefetchNext = false;
-  static constexpr bool kRowConsts = false;
   static constexpr bool kEarlyRelease = false;
   static constexpr bool kTmaStore = false;
   __device__ __forceinline__ void cols(int, const GemmShape&, int, int, uint32_t) const {}
@@ -754,31 +747,24 @@ struct ResBShape {
   uint32_t idesc;
 };
 
-// kEpiWarps = 8 (two warps per TMEM lane quarter, four 32-column chunks each) or 16 (four per quarter, two chunks each:
-// the selection epilogues are bound by the LATENCY of a warp's chunk sequence, not by issue slots -- with four warps per
-// scheduler the sequence is half as long and the other warps fill its bubbles).  kRowSlots: shared-memory slots for
-// Epi::kRowConsts (0 when the epilogue does not use them).
-template <int BN, int kAStages, int kEpiWarps = 8, bool kRowSlots = false, int kStageSlices = 1>
+// kStageSlices: 2 KB staging slices per epilogue warp (two for Epi::kTmaStore: a box is written while the previous drains).
+template <int BN, int kAStages, int kStageSlices = 1>
 struct ResBSmem {
   static constexpr uint32_t kABytes = kBM * kBK * 2;
   static constexpr uint32_t kBPanel = BN * kBK * 2;
   static constexpr uint32_t kMaxKb = 4;
   static constexpr uint32_t kEpiOff = kMaxKb * kBPanel + kAStages * kABytes;
-  static constexpr uint32_t kEpiBytes = kEpiWarps * 2048 * kStageSlices;
-  static constexpr uint32_t kRowConstOff = kEpiOff + kEpiBytes;   // 2 slots x 128 rows x 32 B (Epi::kRowConsts)
-  static constexpr uint32_t kRowConstSlot = kRowSlots ? kBM * 32 : 0;
-  static constexpr uint32_t kBarOff = kRowConstOff + 2 * kRowConstSlot;
-  static constexpr uint32_t kNumBars = 2 * kAStages + 2 + 4 + 2;
+  static constexpr uint32_t kEpiBytes = 8 * 2048 * kStageSlices;
+  static constexpr uint32_t kBarOff = kEpiOff + kEpiBytes;
+  static constexpr uint32_t kNumBars = 2 * kAStages + 2 + 4;
   static constexpr uint32_t kTotal = kBarOff + kNumBars * 8 + 16 + 1024;
 };
 
-template <int BN, int kAStages, class Epi, int kEpiWarps = 8>
-__global__ void __launch_bounds__(128 + 32 * kEpiWarps, 1)
+template <int BN, int kAStages, class Epi>
+__global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_resb_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
                          const ResBShape s, const __grid_constant__ Epi epi) {
-  using L = ResBSmem<BN, kAStages, kEpiWarps, Epi::kRowConsts, Epi::kTmaStore ? 2 : 1>;
-  static_assert(kEpiWarps == 8 || kEpiWarps == 16, "two or four epilogue warps per TMEM lane quarter");
-  static_assert(kEpiWarps == 8 || Epi::kSplitColumns, "four warps per quarter split the tile's columns");
+  using L = ResBSmem<BN, kAStages, Epi::kTmaStore ? 2 : 1>;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_u32 = smem_u32(smem_raw);
   const uint32_t base = (raw_u32 + 1023u) & ~1023u;
@@ -791,8 +777,6 @@ gemm_resb_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid
   const uint32_t b_empty = bar0 + 8u * (2 * kAStages + 1);
   auto tfull_bar = [&](int i) { return bar0 + 8u * (2 * kAStages + 2 + i); };
   auto tempty_bar = [&](int i) { return bar0 + 8u * (2 * kAStages + 4 + i); };
-  auto cfull_bar = [&](int i) { return bar0 + 8u * (2 * kAStages + 6 + i); };       // row constants of tile `it` are in slot it & 1
-  auto cslot = [&](int i) { return base + L::kRowConstOff + i * L::kRowConstSlot; };
   const uint32_t tmem_slot = bar0 + 8u * L::kNumBars;
   volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(smem_raw + (tmem_slot - raw_u32));
   const int warp = threadIdx.x >> 5;
@@ -813,8 +797,7 @@ gemm_resb_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid
     mbar_init(b_empty, 1);
     for (int i = 0; i < 2; ++i) {
       mbar_init(tfull_bar(i), 1);
-      mbar_init(tempty_bar(i), kEpiWarps);
-      mbar_init(cfull_bar(i), 1);
+      mbar_init(tempty_bar(i), 8);
     }
     fence_mbar_init();
   }
@@ -888,35 +871,11 @@ gemm_resb_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid
       }
       tc_commit(b_empty);  // the panel may be overwritten once every MMA of this unit has retired
     }
-  } else if (warp == 3) {
-   if constexpr (Epi::kRowConsts) {
-    // ===================== row-constant prefetcher (the otherwise idle fourth control warp) =====================
-    // Per-row inputs of the epilogue (mining: |a-p|^2, the two excluded guids, the anchor's running bound) are fetched for
-    // tile `it` into shared-memory slot it & 1 as soon as the epilogue has released tile it-2 -- about one tile ahead of
-    // their use.  Loaded by the epilogue warps themselves they sat on the critical path: an epilogue-bound tile starts
-    // with the accumulator already complete, so every tile paid a full L2 round trip before its first instruction.
-    int it = 0;
-    GemmShape gs;
-    gs.M = s.M, gs.N = s.N, gs.K = s.K;
-    for (int u = blockIdx.x; u < units; u += gridDim.x) {
-      const int chunk = s.n_fastest ? u / s.n_tiles : u % s.m_chunks;
-      const int t0 = chunk * s.tiles_per_chunk, t1 = min(s.m_tiles, t0 + s.tiles_per_chunk);
-      for (int t = t0; t < t1; ++t, ++it) {
-        const int as = it & 1;
-        const uint32_t ap = (it >> 1) & 1;
-        mbar_wait(tempty_bar(as), ap ^ 1, 700 + as);
-#pragma unroll
-        for (int r = lane; r < kBM; r += 32) epi.row_consts(t * kBM + r, gs, cslot(as) + r * 32);
-        __syncwarp();
-        if (lane == 0) mbar_arrive(cfull_bar(as));
-      }
-    }
-   }
   } else if (warp >= 4) {
     // ===================== epilogue =====================
     const int q = warp & 3;
-    const int half = (warp - 4) >> 2;         // which share of the tile's columns (0..kEpiWarps/4-1)
-    const uint32_t stg = base + L::kEpiOff + (warp - 4) * (Epi::kTmaStore ? 4096u : (Epi::kSplitColumns || kEpiWarps == 16) ? 2048u : 4096u);
+    const int half = (warp - 4) >> 2;         // which half of the tile's columns
+    const uint32_t stg = base + L::kEpiOff + (warp - 4) * (Epi::kSplitColumns && !Epi::kTmaStore ? 2048u : 4096u);
     int it = 0;
     GemmShape gs;
     gs.M = s.M, gs.N = s.N, gs.K = s.K, gs.m_tiles = s.m_tiles, gs.n_tiles = s.n_tiles, gs.num_kb = s.num_kb;
@@ -940,15 +899,14 @@ gemm_resb_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid
       }
     };
     const bool active = Epi::kSplitColumns || half == 0;
-    constexpr int kChunksPerWarp = (BN / 32) / (kEpiWarps / 4);
-    const int ec0 = Epi::kSplitColumns ? half * kChunksPerWarp : 0, ec1 = Epi::kSplitColumns ? (half + 1) * kChunksPerWarp : BN / 32;
+    const int ec0 = Epi::kSplitColumns ? half * (BN / 64) : 0, ec1 = Epi::kSplitColumns ? (half + 1) * (BN / 64) : BN / 32;
     TileIter cur;
     cur.u = blockIdx.x;
     seek(cur);
     typename Epi::State est;
     if (cur.valid && active) {
       epi.cols(cur.nblk * BN, gs, ec0, ec1, stg);
-      if constexpr (!Epi::kRowConsts) epi.pre(est, cur.t * kBM + q * 32 + lane, cur.nblk * BN, gs, ec0, ec1, stg);
+      epi.pre(est, cur.t * kBM + q * 32 + lane, cur.nblk * BN, gs, ec0, ec1, stg);
     }
     while (cur.valid) {
       TileIter nxt = cur;
@@ -959,17 +917,11 @@ gemm_resb_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid
       const int as = it & 1;
       const uint32_t ap = (it >> 1) & 1;
       typename Epi::State est_next;
-      if constexpr (Epi::kRowConsts) {
-        mbar_wait(cfull_bar(as), ap, 800 + as);
-        if (active) epi.load_state(est, cslot(as) + (q * 32 + lane) * 32);
-        est_next = est;
-      }
       mbar_wait(tfull_bar(as), ap, 400 + as);
       tc_fence_after();
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + as * BN;
       if (active) {
-        if constexpr (!Epi::kRowConsts)
-          if (Epi::kPrefetchNext && nxt.valid) epi.pre(est_next, nxt.t * kBM + q * 32 + lane, nxt.nblk * BN, gs, ec0, ec1, stg);
+        if (Epi::kPrefetchNext && nxt.valid) epi.pre(est_next, nxt.t * kBM + q * 32 + lane, nxt.nblk * BN, gs, ec0, ec1, stg);
         // kEarlyRelease: the epilogue hands the accumulator buffer back itself, right after its LAST TMEM read (it still
         // has that chunk to process from registers): the MMA of the tile after next starts that much earlier
         if constexpr (Epi::kEarlyRelease) est.release_bar = tempty_bar(as);
@@ -982,8 +934,7 @@ gemm_resb_tcgen05_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid
       }
       if (active && nxt.valid) {
         epi.cols(nxt.nblk * BN, gs, ec0, ec1, stg);   // the previous tile no longer reads the column cache
-        if constexpr (!Epi::kRowConsts)
-          if (!Epi::kPrefetchNext) epi.pre(est_next, nxt.t * kBM + q * 32 + lane, nxt.nblk * BN, gs, ec0, ec1, stg);
+        if (!Epi::kPrefetchNext) epi.pre(est_next, nxt.t * kBM + q * 32 + lane, nxt.nblk * BN, gs, ec0, ec1, stg);
       }
       est = est_next;
       cur = nxt;

@@ -47,7 +47,6 @@ template <int BN>
 struct EpiKnnGroupMax {
   static constexpr bool kSplitColumns = true;
   static constexpr bool kPrefetchNext = false;
-  static constexpr bool kRowConsts = false;
   static constexpr bool kEarlyRelease = false;
   static constexpr bool kTmaStore = false;
   struct State {};
@@ -124,7 +123,6 @@ struct EpiKnnCollect {
     uint32_t release_bar;   // resident-B kernel: the accumulator buffer's "empty" barrier (0: the kernel arrives itself)
   };
   static constexpr bool kPrefetchNext = true;   // pre() only loads a row constant into registers
-  static constexpr bool kRowConsts = false;
   static constexpr bool kEarlyRelease = true;
   static constexpr bool kTmaStore = false;
   __device__ __forceinline__ void block_begin(uint32_t epi_smem) const {

@@ -15,61 +15,83 @@ namespace cdml {
 constexpr unsigned long long kNoCand = ~0ull;
 constexpr int kMassHits = 4;   // rows of a warp hitting in one chunk from which the per-thread re-scan takes over
 
-// epilogue warps of the mining scans: 8 (two per TMEM lane quarter).  CDML_MINE_EPI_WARPS=16 selects four per quarter (A/B
-// measurement aid): measured on B200 it is SLOWER (4.28 vs 4.02 ms structureless, 4.24 vs 3.94 ms clustered for both scans) --
-// the epilogue is not short of warps; see DESIGN.md section 4.4
-static int epi_warps() {
-  static int w = -1;
-  if (w < 0) {
-    const char* e = getenv("CDML_MINE_EPI_WARPS");
-    w = (e != nullptr && e[0] == '1') ? 16 : 8;
+// What the two selection epilogues (EpiMine, EpiMineDW) share: the candidate set of one launch, the traits, the column
+// cache of candidate guids, the pipelined TMEM reads of a warp's four 32-column chunks, and the staging of one row's 32
+// scores for the cooperative re-scan.  The per-chunk selection is the mode's own.
+struct EpiMineBase {
+  static constexpr bool kSplitColumns = true;
+  static constexpr bool kPrefetchNext = false;   // pre() only loads the anchor's constants into registers
+  static constexpr bool kEarlyRelease = true;
+  static constexpr bool kTmaStore = false;
+  const float* dp;        // [B] exact |a-p|^2
+  const int32_t* guid;    // [B,3] int32 guids
+  unsigned long long* best;  // [B] 64-bit key per anchor: (32-bit order key of the pick) << 32 | row
+  int cand;  // 1: columns are the positives' rows 3j+1, 2: the negatives' rows 3j+2
+  unsigned long long* stats;   // [0] += re-scanned (anchor, 32-column chunk) pairs
+  // candidate guids of the warp's 128 columns, once per column block (-1 beyond N: the re-scan skips them)
+  __device__ __forceinline__ void cols(int n0, const GemmShape& s, int c0, int /*c1*/, uint32_t stg) const {
+    col_cache_fill(stg, n0, c0, [&](int col) { return static_cast<uint32_t>(col < s.N ? __ldg(guid + 3 * col + cand) : -1); });
   }
-  return w;
-}
+  __device__ __forceinline__ void block_begin(uint32_t epi_smem) const { col_cache_reset(epi_smem); }
+  __device__ __forceinline__ void block_end(uint32_t) const {}
+  // candidate guid of column j of chunk cc (column cache)
+  static __device__ __forceinline__ int cand_guid(uint32_t stg, int cc, int j) {
+    int g;
+    asm volatile("ld.shared.b32 %0, [%1];" : "=r"(g) : "r"(stg + kColCacheOff + 128 * cc + 4 * j) : "memory");
+    return g;
+  }
+  // Row src's 32 scores through the warp's staging slice: lane j gets column j.
+  static __device__ __forceinline__ float stage_row(uint32_t stg, const uint32_t (&v)[32], int src) {
+    __syncwarp();
+    if ((threadIdx.x & 31) == src) {
+#pragma unroll
+      for (int j = 0; j < 8; ++j) sts128(stg + 16 * j, v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+    }
+    __syncwarp();
+    float sc;
+    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(sc) : "r"(stg + 4 * (threadIdx.x & 31)) : "memory");
+    return sc;
+  }
+  // chunk(v, cc) for each of the warp's chunks inside the tile and the matrix, TMEM reads double-buffered.  release_bar
+  // != 0 (resident-B kernel): the accumulator buffer is handed back as soon as the warp's last read has landed, before
+  // the last chunk is processed.
+  template <class Chunk>
+  static __device__ __forceinline__ void scan(uint32_t taddr, int n0, const GemmShape& s, int c0, int c1,
+                                              uint32_t release_bar, Chunk&& chunk) {
+    uint32_t va[32], vb[32];
+    auto ok = [&](int cc) { return c0 + cc < c1 && n0 + (c0 + cc) * 32 < s.N; };   // warp-uniform
+    tmem_ld_32x32(taddr + c0 * 32, va);
+#pragma unroll
+    for (int cc = 0; cc < 4; cc += 2) {
+      tmem_ld_wait();
+      if (ok(cc + 1)) tmem_ld_32x32(taddr + (c0 + cc + 1) * 32, vb);
+      if (ok(cc)) chunk(va, cc);
+      tmem_ld_wait();
+      if (cc + 2 < 4 && ok(cc + 2)) tmem_ld_32x32(taddr + (c0 + cc + 2) * 32, va);
+      if (cc + 2 >= 4 && release_bar != 0u) {   // every TMEM read of this warp has landed: release the buffer now
+        tc_fence_before();
+        __syncwarp();
+        if ((threadIdx.x & 31) == 0) mbar_arrive(release_bar);
+      }
+      if (ok(cc + 1)) chunk(vb, cc + 1);
+    }
+  }
+};
 
 // (1)/(2) collapse into ONE criterion: the chosen row is argmin d over valid candidates with d > dp -- if that minimum
 // is below dp+margin it is the semi-hard pick, otherwise it is exactly the closest beyond-margin pick.
 // Common path per score: d = 2-2s, keep min over (d > dp).  Only when a 32-column chunk can beat the anchor's current
 // best (a bound read from the global key at tile start; rare after the first tiles) are guids checked and the row
 // recorded.  Result: 64-bit key (float bits of d << 32 | row) folded with atomicMin -> ties go to the lowest row.
-template <int BN, int kVariant = 0>
-struct EpiMine {
-  static constexpr bool kSplitColumns = true;
-  static constexpr bool kPrefetchNext = (kVariant & 1) == 0;   // pre() only loads the anchor's constants into registers
-  // resident-B kernel: the anchor's four constants arrive through shared memory, fetched one tile ahead by the spare
-  // control warp (row_consts / load_state); the generic kernel (small batches) still calls pre()
-  static constexpr bool kRowConsts = (kVariant & 4) != 0;   // measured on B200: no gain (3.93 vs 3.89 ms clustered) and the
-                                                             // two-tile-old bound costs re-scans (5.0 vs 4.3 ms structureless)
+template <int BN>
+struct EpiMine : EpiMineBase {
+  static_assert(BN == 256, "a warp owns 4 chunks (128 columns) of the tile");
   struct State {
     float dpi, bound_d;
     int ga, gp;
     uint32_t bound_row;   // row of the anchor's best candidate so far (ties -> lowest row)
     uint32_t release_bar; // resident-B kernel: the accumulator buffer's "empty" barrier (0: the kernel arrives itself)
   };
-  static constexpr bool kEarlyRelease = true;
-  static constexpr bool kTmaStore = false;
-  const float* dp;        // [B] exact |a-p|^2
-  const int32_t* guid;    // [B,3] int32 guids
-  unsigned long long* best;  // [B] (float bits of d) << 32 | row
-  int cand;  // 1: columns are the positives' rows 3j+1, 2: the negatives' rows 3j+2
-  unsigned long long* stats;   // [0] += re-scanned (anchor, 32-column chunk) pairs
-  __device__ __forceinline__ void row_consts(int row, const GemmShape& s, uint32_t dst) const {
-    const bool row_ok = row < s.M;
-    const uint32_t inf = 0x7f800000u;
-    const uint32_t dpi = row_ok ? __float_as_uint(__ldg(dp + row)) : inf;
-    const uint32_t ga = row_ok ? static_cast<uint32_t>(__ldg(guid + 3 * row)) : 0u;
-    const uint32_t gp = row_ok ? static_cast<uint32_t>(__ldg(guid + 3 * row + 1)) : 0u;
-    const unsigned long long key = row_ok ? *(reinterpret_cast<volatile unsigned long long*>(best) + row) : ~0ull;
-    sts128(dst, dpi, ga, gp, static_cast<uint32_t>(key >> 32));
-    asm volatile("st.shared.b32 [%0], %1;" ::"r"(dst + 16), "r"(static_cast<uint32_t>(key)) : "memory");
-  }
-  __device__ __forceinline__ void load_state(State& st, uint32_t src) const {
-    const uint4 v = lds128(src);
-    st.dpi = __uint_as_float(v.x), st.ga = static_cast<int>(v.y), st.gp = static_cast<int>(v.z), st.bound_d = __uint_as_float(v.w);
-    asm volatile("ld.shared.b32 %0, [%1];" : "=r"(st.bound_row) : "r"(src + 16) : "memory");
-    st.release_bar = 0u;
-  }
-  // the anchor's constants do not depend on the accumulator: the resident-B kernel issues them one tile ahead
   __device__ __forceinline__ void pre(State& st, int row, int /*n0*/, const GemmShape& s, int, int, uint32_t) const {
     const bool row_ok = row < s.M;
     const float inf = __int_as_float(0x7f800000);
@@ -81,13 +103,6 @@ struct EpiMine {
     st.bound_row = static_cast<uint32_t>(key);
     st.release_bar = 0u;
   }
-  // candidate guids of the warp's 128 columns, once per column block (-1 beyond N: the re-scan skips them)
-  __device__ __forceinline__ void cols(int n0, const GemmShape& s, int c0, int /*c1*/, uint32_t stg) const {
-    static_assert(BN == 256, "a warp owns 4 chunks (128 columns) of the tile");
-    col_cache_fill(stg, n0, c0, [&](int col) { return static_cast<uint32_t>(col < s.N ? __ldg(guid + 3 * col + cand) : -1); });
-  }
-  __device__ __forceinline__ void block_begin(uint32_t epi_smem) const { col_cache_reset(epi_smem); }
-  __device__ __forceinline__ void block_end(uint32_t) const {}
   // Works in score space: d = 2 - 2s, so "d > dp" is "s < s_hi" and the closest candidate is the LARGEST such score.
   __device__ __forceinline__ void run(uint32_t taddr, int row, int n0, int /*split*/, const GemmShape& s, int c0,
                                       int c1, uint32_t stg, State& st) const {
@@ -103,7 +118,6 @@ struct EpiMine {
     uint32_t brow = st.bound_row;                              // ... and a score EQUAL to it only in a row below this one
     float bd = inf;
     int br = -1;
-    uint32_t va[32], vb[32];
     auto chunk = [&](const uint32_t (&v)[32], int cc) {
       const int nb = n0 + (c0 + cc) * 32;
       // Hot loop, one instruction per score: t = s_hi - score in packed fp32x2 subtracts, then a 3-input UNSIGNED
@@ -139,8 +153,7 @@ struct EpiMine {
           int cbest = -1;
 #pragma unroll
           for (int j = 0; j < 32; ++j) {
-            int g;
-            asm volatile("ld.shared.b32 %0, [%1];" : "=r"(g) : "r"(stg + kColCacheOff + 128 * cc + 4 * j) : "memory");
+            const int g = cand_guid(stg, cc, j);
             const float sc = __uint_as_float(v[j]);
             const float d = fmaxf(fmaf(-2.f, sc, 2.f), 0.f);
             const bool pass = sc < s_hi && sc >= s_lo && d > dpi && d < bd && g != ga && g != gp && g >= 0;
@@ -156,19 +169,11 @@ struct EpiMine {
         __syncwarp();
       } else if (hits != 0u) {
         if (lane == 0) atomicAdd(stats, static_cast<unsigned long long>(__popc(hits)));
-        int g_lane;   // candidate guid of column nb + lane (column cache)
-        asm volatile("ld.shared.b32 %0, [%1];" : "=r"(g_lane) : "r"(stg + kColCacheOff + 128 * cc + 4 * lane) : "memory");
+        const int g_lane = cand_guid(stg, cc, lane);   // candidate guid of column nb + lane
         do {
           const int src = __ffs(hits) - 1;
           hits &= hits - 1u;
-          __syncwarp();
-          if (lane == src) {
-#pragma unroll
-            for (int j = 0; j < 8; ++j) sts128(stg + 16 * j, v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-          }
-          __syncwarp();
-          float sc;
-          asm volatile("ld.shared.f32 %0, [%1];" : "=f"(sc) : "r"(stg + 4 * lane) : "memory");
+          const float sc = stage_row(stg, v, src);
           const float hi_s = __shfl_sync(0xffffffffu, s_hi, src), lo_s = __shfl_sync(0xffffffffu, s_lo, src);
           const float dp_s = __shfl_sync(0xffffffffu, dpi, src), bd_s = __shfl_sync(0xffffffffu, bd, src);
           const int ga_s = __shfl_sync(0xffffffffu, ga, src), gp_s = __shfl_sync(0xffffffffu, gp, src);
@@ -187,38 +192,7 @@ struct EpiMine {
         } while (hits != 0u);
       }
     };
-    auto ok = [&](int cc) { return c0 + cc < c1 && n0 + (c0 + cc) * 32 < s.N; };   // warp-uniform
-    if constexpr ((kVariant & 2) == 0) {
-      tmem_ld_32x32(taddr + c0 * 32, va);
-#pragma unroll
-      for (int cc = 0; cc < 4; cc += 2) {
-        tmem_ld_wait();
-        if (ok(cc + 1)) tmem_ld_32x32(taddr + (c0 + cc + 1) * 32, vb);
-        if (ok(cc)) chunk(va, cc);
-        tmem_ld_wait();
-        if (cc + 2 < 4 && ok(cc + 2)) tmem_ld_32x32(taddr + (c0 + cc + 2) * 32, va);
-        if (cc + 2 >= 4 && st.release_bar != 0u) {   // every TMEM read of this warp has landed: release the buffer now
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(st.release_bar);
-        }
-        if (ok(cc + 1)) chunk(vb, cc + 1);
-      }
-    } else {
-#pragma unroll
-      for (int cc = 0; cc < 4; ++cc) {
-        if (ok(cc)) {
-          tmem_ld_32x32(taddr + (c0 + cc) * 32, va);
-          tmem_ld_wait();
-          chunk(va, cc);
-        }
-      }
-      if (st.release_bar != 0u) {
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(st.release_bar);
-      }
-    }
+    scan(taddr, n0, s, c0, c1, st.release_bar, chunk);
     if (br >= 0)
       atomicMin(best + row, (static_cast<unsigned long long>(__float_as_uint(bd)) << 32) | static_cast<uint32_t>(br));
   }
@@ -247,23 +221,14 @@ __device__ __forceinline__ float dw_exp1(uint32_t x) {   // accurate log: relati
 }
 
 template <int BN>
-struct EpiMineDW {
-  static constexpr bool kSplitColumns = true;
-  static constexpr bool kPrefetchNext = false;
-  static constexpr bool kRowConsts = false;
-  static constexpr bool kEarlyRelease = true;
-  static constexpr bool kTmaStore = false;
+struct EpiMineDW : EpiMineBase {
+  static_assert(BN == 256, "a warp owns 4 chunks (128 columns) of the tile");
   struct State {
     float dpm;            // dp + margin: eligible iff delta < dpm
     int ga, gp;
     uint32_t bkey, brow;  // the anchor's best (key, row) so far, from the global key at tile start
     uint32_t release_bar;
   };
-  const float* dp;
-  const int32_t* guid;
-  unsigned long long* best;  // [B] f2key(key) << 32 | row
-  int cand;
-  unsigned long long* stats;
   float margin, dmin, ha, hb;   // dmin = cutoff^2, ha = (D-2)/2, hb = (D-3)/2
   uint32_t seed_lo, seed_hi;
   const int64_t* step;          // device step counter (nullptr: 0), read at every launch so graph replays draw anew
@@ -279,12 +244,6 @@ struct EpiMineDW {
     st.bkey = static_cast<uint32_t>(key >> 32), st.brow = static_cast<uint32_t>(key);
     st.release_bar = 0u;
   }
-  __device__ __forceinline__ void cols(int n0, const GemmShape& s, int c0, int /*c1*/, uint32_t stg) const {
-    static_assert(BN == 256, "a warp owns 4 chunks (128 columns) of the tile");
-    col_cache_fill(stg, n0, c0, [&](int col) { return static_cast<uint32_t>(col < s.N ? __ldg(guid + 3 * col + cand) : -1); });
-  }
-  __device__ __forceinline__ void block_begin(uint32_t epi_smem) const { col_cache_reset(epi_smem); }
-  __device__ __forceinline__ void block_end(uint32_t) const {}
   __device__ __forceinline__ void run(uint32_t taddr, int row, int n0, int /*split*/, const GemmShape& s, int c0,
                                       int c1, uint32_t stg, State& st) const {
     const int lane = threadIdx.x & 31;
@@ -297,7 +256,6 @@ struct EpiMineDW {
     bool found = false;
     const uint64_t stp = step != nullptr ? static_cast<uint64_t>(__ldg(step)) : 0ull;
     const uint32_t ctr2 = static_cast<uint32_t>(stp), ctr3 = static_cast<uint32_t>(stp >> 32) << 4;
-    uint32_t va[32], vb[32];
     // exact key of column j's score sc given its draw word x (unused for j == K); +inf when not eligible
     auto key_of = [&](float sc, int j, uint32_t x, float M, uint32_t K, float dpm_, int g, int ga_, int gp_) {
       const float delta = fmaxf(fmaf(-2.f, sc, 2.f), dmin);
@@ -346,8 +304,7 @@ struct EpiMineDW {
 #pragma unroll
             for (int t = 0; t < 4; ++t) {
               const int j = 4 * w + t;
-              int g;
-              asm volatile("ld.shared.b32 %0, [%1];" : "=r"(g) : "r"(stg + kColCacheOff + 128 * cc + 4 * j) : "memory");
+              const int g = cand_guid(stg, cc, j);
               const uint32_t k = key_of(__uint_as_float(v[j]), j, xs[t], M, K, dpm, g, ga, gp);
               if (k < kbest) kbest = k, cbest = j;
             }
@@ -357,19 +314,11 @@ struct EpiMineDW {
         }
         __syncwarp();
       } else {
-        int g_lane;   // candidate guid of column nb + lane (column cache)
-        asm volatile("ld.shared.b32 %0, [%1];" : "=r"(g_lane) : "r"(stg + kColCacheOff + 128 * cc + 4 * lane) : "memory");
+        const int g_lane = cand_guid(stg, cc, lane);   // candidate guid of column nb + lane
         do {   // one hitting row at a time: lane j evaluates column j (its draw is word j % 4 of call 1 + j / 4)
           const int src = __ffs(hits) - 1;
           hits &= hits - 1u;
-          __syncwarp();
-          if (lane == src) {
-#pragma unroll
-            for (int j = 0; j < 8; ++j) sts128(stg + 16 * j, v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-          }
-          __syncwarp();
-          float sc;
-          asm volatile("ld.shared.f32 %0, [%1];" : "=f"(sc) : "r"(stg + 4 * lane) : "memory");
+          const float sc = stage_row(stg, v, src);
           const int row_s = __shfl_sync(0xffffffffu, row, src);
           const float M_s = __shfl_sync(0xffffffffu, M, src), dpm_s = __shfl_sync(0xffffffffu, dpm, src);
           const uint32_t K_s = __shfl_sync(0xffffffffu, K, src);
@@ -387,22 +336,7 @@ struct EpiMineDW {
         } while (hits != 0u);
       }
     };
-    auto ok = [&](int cc) { return c0 + cc < c1 && n0 + (c0 + cc) * 32 < s.N; };   // warp-uniform
-    tmem_ld_32x32(taddr + c0 * 32, va);
-#pragma unroll
-    for (int cc = 0; cc < 4; cc += 2) {
-      tmem_ld_wait();
-      if (ok(cc + 1)) tmem_ld_32x32(taddr + (c0 + cc + 1) * 32, vb);
-      if (ok(cc)) chunk(va, cc);
-      tmem_ld_wait();
-      if (cc + 2 < 4 && ok(cc + 2)) tmem_ld_32x32(taddr + (c0 + cc + 2) * 32, va);
-      if (cc + 2 >= 4 && st.release_bar != 0u) {   // every TMEM read of this warp has landed: release the buffer now
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(st.release_bar);
-      }
-      if (ok(cc + 1)) chunk(vb, cc + 1);
-    }
+    scan(taddr, n0, s, c0, c1, st.release_bar, chunk);
     if (found) atomicMin(best + row, (static_cast<unsigned long long>(bkey) << 32) | brow);
   }
 };
@@ -454,17 +388,12 @@ __global__ void mine_finalize_kernel(const float* __restrict__ E, int64_t ld, in
   if (lane == 0 && mined != 0u) atomicAdd(stats + 1, static_cast<unsigned long long>(mined));
 }
 
-}  // namespace cdml
-
-using namespace cdml;
-
-extern "C" int cdml_mine_semihard(cdml_ctx* ctx, const void* E16, int64_t ld16, int dtype16, const float* E32,
-                                  int64_t ld32, const int64_t* guid, int64_t B, int D, float margin, int32_t* neg_row,
-                                  float* d_an, void* stream) {
-  CDML_REQUIRE(ctx && E16 && E32 && guid && neg_row, "cdml_mine_semihard: NULL argument");
-  CDML_REQUIRE(B > 0 && 3 * B < (1ll << 31) && D > 0 && D % 8 == 0 && ld16 >= D && ld32 >= D,
-               "cdml_mine_semihard: bad geometry B=%lld D=%d", (long long)B, D);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+// Host side of both mining modes: scratch, prepare, one scan per candidate set (positives, then negatives), finalize.
+// make_epi(EpiMineBase) returns the mode's selection epilogue for one scan.
+template <class MakeEpi>
+static int mine_scans(cdml_ctx* ctx, const void* E16, int64_t ld16, int dtype16, const float* E32, int64_t ld32,
+                      const int64_t* guid, int64_t B, int D, int32_t* neg_row, float* d_an, cudaStream_t st,
+                      MakeEpi&& make_epi) {
   // scratch: best [B] u64 | dp [B] f32 | guid32 [3B] i32
   const size_t bytes = static_cast<size_t>(B) * (8 + 4 + 12) + 64;
   uint8_t* ws = static_cast<uint8_t*>(ctx_scratch(ctx, bytes));
@@ -480,17 +409,8 @@ extern "C" int cdml_mine_semihard(cdml_ctx* ctx, const void* E16, int64_t ld16, 
   const uint16_t* e16 = static_cast<const uint16_t*>(E16);
   for (int cand = 1; cand <= 2 && rc >= 0; ++cand) {
     // A: anchors = rows 0,3,6,.. (pitch 3*ld16); B: candidates = rows cand, cand+3, .. ; both K-major, K = D.
-    // Variant 1 (measured best of the four on B200: 3.79 ms vs 4.17-4.25): pipelined TMEM reads, anchor constants
-    // fetched after the previous tile is released (a one-tile-ahead fetch of the running bound makes it staler).
-    EpiMine<kBN, 1> epi{dp, guid32, best, cand, stats};
-    static int rowc = -1;   // CDML_MINE_ROWCONSTS=1: anchor constants through the spare warp's shared-memory slots (A/B aid)
-    if (rowc < 0) rowc = getenv("CDML_MINE_ROWCONSTS") != nullptr ? 1 : 0;
-    if (resb_applicable(D) && B >= 8 * kBM && rowc) {
-      EpiMine<kBN, 5> epi5{dp, guid32, best, cand, stats};
-      rc = launch_gemm_resb(ctx, e16, 3 * ld16, e16 + cand * ld16, 3 * ld16, B, B, D, dtype16, epi5, st);
-    } else if (resb_applicable(D) && B >= 8 * kBM && epi_warps() == 16)
-      rc = launch_gemm_resb<EpiMine<kBN, 1>, 16>(ctx, e16, 3 * ld16, e16 + cand * ld16, 3 * ld16, B, B, D, dtype16, epi, st);
-    else if (resb_applicable(D) && B >= 8 * kBM)
+    const auto epi = make_epi(EpiMineBase{dp, guid32, best, cand, stats});
+    if (resb_applicable(D) && B >= 8 * kBM)
       rc = launch_gemm_resb(ctx, e16, 3 * ld16, e16 + cand * ld16, 3 * ld16, B, B, D, dtype16, epi, st);
     else
       rc = launch_gemm<0, 0>(ctx, e16, 3 * ld16, e16 + cand * ld16, 3 * ld16, B, B, D, dtype16, 1, epi, st);
@@ -502,6 +422,20 @@ extern "C" int cdml_mine_semihard(cdml_ctx* ctx, const void* E16, int64_t ld16, 
   return rc < 0 ? rc : 0;
 }
 
+}  // namespace cdml
+
+using namespace cdml;
+
+extern "C" int cdml_mine_semihard(cdml_ctx* ctx, const void* E16, int64_t ld16, int dtype16, const float* E32,
+                                  int64_t ld32, const int64_t* guid, int64_t B, int D, float margin, int32_t* neg_row,
+                                  float* d_an, void* stream) {
+  CDML_REQUIRE(ctx && E16 && E32 && guid && neg_row, "cdml_mine_semihard: NULL argument");
+  CDML_REQUIRE(B > 0 && 3 * B < (1ll << 31) && D > 0 && D % 8 == 0 && ld16 >= D && ld32 >= D,
+               "cdml_mine_semihard: bad geometry B=%lld D=%d", (long long)B, D);
+  return mine_scans(ctx, E16, ld16, dtype16, E32, ld32, guid, B, D, neg_row, d_an, static_cast<cudaStream_t>(stream),
+                    [](const EpiMineBase& c) { return EpiMine<kBN>{c}; });
+}
+
 extern "C" int cdml_mine_distance_weighted(cdml_ctx* ctx, const void* E16, int64_t ld16, int dtype16, const float* E32,
                                            int64_t ld32, const int64_t* guid, int64_t B, int D, float margin, float cutoff,
                                            uint64_t seed, const int64_t* step, int32_t* neg_row, float* d_an,
@@ -511,32 +445,11 @@ extern "C" int cdml_mine_distance_weighted(cdml_ctx* ctx, const void* E16, int64
                "cdml_mine_distance_weighted: bad geometry B=%lld D=%d", (long long)B, D);
   CDML_REQUIRE(cutoff > 0.f && cutoff < 2.f && margin == margin, "cdml_mine_distance_weighted: cutoff %g not in (0, 2)",
                (double)cutoff);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const size_t bytes = static_cast<size_t>(B) * (8 + 4 + 12) + 64;   // as cdml_mine_semihard
-  uint8_t* ws = static_cast<uint8_t*>(ctx_scratch(ctx, bytes));
-  if (ws == nullptr) return -2;
-  if (ctx->mine_stats == nullptr) CDML_CHECK_CUDA(cudaMalloc(&ctx->mine_stats, 2 * sizeof(unsigned long long)));
-  unsigned long long* stats = ctx->mine_stats;
-  unsigned long long* best = reinterpret_cast<unsigned long long*>(ws);
-  float* dp = reinterpret_cast<float*>(best + B);
-  int32_t* guid32 = reinterpret_cast<int32_t*>(dp + B);
-  const int grid = static_cast<int>(std::min<int64_t>((B + 7) / 8, ctx->num_sms * 8));
-  mine_prepare_kernel<<<grid, 256, 0, st>>>(E32, ld32, D, guid, B, dp, guid32, best, stats);
-  int rc = 0;
-  const uint16_t* e16 = static_cast<const uint16_t*>(E16);
-  for (int cand = 1; cand <= 2 && rc >= 0; ++cand) {
-    EpiMineDW<kBN> epi{dp, guid32, best, cand, stats, margin, cutoff * cutoff, 0.5f * (D - 2), 0.5f * (D - 3),
-                       static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32), step};
-    if (resb_applicable(D) && B >= 8 * kBM)
-      rc = launch_gemm_resb(ctx, e16, 3 * ld16, e16 + cand * ld16, 3 * ld16, B, B, D, dtype16, epi, st);
-    else
-      rc = launch_gemm<0, 0>(ctx, e16, 3 * ld16, e16 + cand * ld16, 3 * ld16, B, B, D, dtype16, 1, epi, st);
-  }
-  if (rc >= 0) {
-    mine_finalize_kernel<<<grid, 256, 0, st>>>(E32, ld32, D, best, B, neg_row, d_an, stats);
-    rc = cudaGetLastError() == cudaSuccess ? 0 : -2;
-  }
-  return rc < 0 ? rc : 0;
+  return mine_scans(ctx, E16, ld16, dtype16, E32, ld32, guid, B, D, neg_row, d_an, static_cast<cudaStream_t>(stream),
+                    [&](const EpiMineBase& c) {
+                      return EpiMineDW<kBN>{c, margin, cutoff * cutoff, 0.5f * (D - 2), 0.5f * (D - 3),
+                                            static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32), step};
+                    });
 }
 
 extern "C" int cdml_mine_last_stats(cdml_ctx* ctx, int64_t* out2, void* stream) {

@@ -71,7 +71,6 @@ class TowerEngine:
     self.F_pad = _pad64(self.F + 1)     # always one spare column: it carries the ones of [x | 1] (bias gradient row)
     self.loss_scale = 1.0          # multiplies the 16-bit backward signal; divided out inside the optimizer kernel's grad_scale
     self.fused_bias_grad = True    # bias gradients as an extra row of the weight-gradient GEMMs (no colsum kernels)
-    self.ddp_buckets = os.environ.get("CDML_DDP_BUCKETS", "0") == "1"
     self._ones_checked = {}
 
     # ---- flat fp32 parameter / gradient / Adam buffers; per-tensor views ----
@@ -311,18 +310,10 @@ class TowerEngine:
 
   def backward_rows(self, x16, R, buf, input_ones=False):
     dz = buf["dz"]
-    self._pending = []
     for l in range(self.L - 1, -1, -1):
       K_in, N_out = self.dims[l], self.dims[l + 1]
       inp = x16 if l == 0 else buf["acts"][l - 1]
       self._weight_gradient(l, inp, dz[l], R, buf, with_bias_row=(l > 0 or input_ones))
-      if self.world > 1 and self.ddp_buckets and l > 0:
-        # bucketed exchange: [dW_l ; db_l] is complete -- its all-reduce may run (on NCCL's stream) under the data-gradient
-        # and weight-gradient GEMMs of the layers below.  Off by default: the GEMMs are persistent kernels that own every
-        # SM (one CTA of ~215 KB shared memory and ~56K registers per SM), so a concurrent NCCL kernel only gets SMs
-        # when a GEMM CTA retires -- measured no gain (DESIGN.md section 5)
-        o0, o1 = int(self.offsets[2 * l]), int(self.offsets[2 * l + 2])
-        self._pending.append(torch.distributed.all_reduce(self.g[o0:o1], group=self.pg, async_op=True))
       if l > 0:
         # data gradient + leaky' of the previous layer: dz[l-1] = (dz[l] . W_l^T) * leaky'(h_{l-1})
         ops.gemm16(dz[l], self.W16[l], R, K_in, N_out, 0, 0, EPI_MASK_BITS, dz[l - 1], alpha=self.alpha,
@@ -347,14 +338,7 @@ class TowerEngine:
 
   def apply_gradients(self, B_local):
     if self.world > 1:
-      pending = getattr(self, "_pending", [])
-      if pending:                      # layers >= 1 are already in flight; layer 0's block follows and all are awaited
-        torch.distributed.all_reduce(self.g[:int(self.offsets[2])], group=self.pg)
-        for w in pending:
-          w.wait()
-        self._pending = []
-      else:
-        torch.distributed.all_reduce(self.g, group=self.pg)  # NCCL sum over ranks, one flat buffer
+      torch.distributed.all_reduce(self.g, group=self.pg)  # NCCL sum over ranks, one flat buffer
     ops.adam_prepare(self.step_counter, self.scalars, self.base_lr, self.lr_decay_steps, self.lr_decay, True,
                      self.beta1, self.beta2)
     scale = 1.0 / (B_local * self.world * self.loss_scale)

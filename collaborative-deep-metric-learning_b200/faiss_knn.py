@@ -78,15 +78,6 @@ def sharded_search(index, xq, k, id_offset=0, metric="L2", process_group=None, m
   if not hasattr(index, "shard_bounds"):
     return _sharded_search_lists(index, xq, k, id_offset, metric, process_group, merge_fn)
   deferred = merge_packed_fn is None and not _sync_refine       # (the CPU stand-in of the gloo test has no deferred mode)
-  if deferred and xq.is_cuda and os.environ.get("CDML_KNN_GRAPH", "0") == "1":
-    # EXPERIMENTAL, off by default (CDML_KNN_GRAPH=1): the whole protocol -- ~20 kernel launches and five collectives --
-    # replayed as ONE CUDA graph per (query count, k).  Measured on 2 GPUs: same time as the eager deferred form (20.8 ms
-    # per 65 536 queries, the ranks are not launch-bound there), ids identical; a four-chunk block (262 144 queries) of
-    # tools/cycle.py did not complete under it -- not yet understood, hence not the product path.
-    out, overflowed = _graph_sharded(index, xq, k, id_offset, metric, process_group, gather)
-    if not overflowed:
-      return out
-    return sharded_search(index, xq, k, id_offset, metric, process_group, merge_fn, gather, merge_packed_fn, _sync_refine=True)
   out, flag = _run_sharded(index, xq, k, id_offset, metric, process_group, gather, deferred, merge_packed_fn)
   if flag is not None and int(flag.item()) != 0:             # some shard overflowed somewhere: redo with the exact fallback (rare)
     return sharded_search(index, xq, k, id_offset, metric, process_group, merge_fn, gather, merge_packed_fn, _sync_refine=True)
@@ -94,8 +85,8 @@ def sharded_search(index, xq, k, id_offset=0, metric="L2", process_group=None, m
 
 
 def _run_sharded(index, xq, k, id_offset, metric, process_group, gather, deferred, merge_packed_fn=None):
-  """One pass of the record protocol, enqueued on the current stream (capturable when `deferred`).  Returns ((D, I), flag):
-  flag is the device word agreed over the ranks (None in the synchronous form)."""
+  """One pass of the record protocol, enqueued on the current stream without a host round trip when `deferred`.  Returns
+  ((D, I), flag): flag is the device word agreed over the ranks (None in the synchronous form)."""
   dist = torch.distributed
   world = dist.get_world_size(process_group)
   nq = xq.shape[0]
@@ -134,35 +125,6 @@ def _run_sharded(index, xq, k, id_offset, metric, process_group, gather, deferre
   if flag is not None:
     dist.all_reduce(flag, op=dist.ReduceOp.MAX, group=process_group)
   return out, flag
-
-
-def _graph_sharded(index, xq, k, id_offset, metric, process_group, gather):
-  """Capture-once / replay form of _run_sharded.  Every rank must call it with the same shapes in the same order (SPMD, like
-  every collective).  Returns ((D, I) copies, overflowed)."""
-  graphs = index.__dict__.setdefault("_shard_graphs", {})
-  key = (tuple(xq.shape), int(k), metric, bool(gather), int(id_offset), id(process_group))
-  g = graphs.get(key)
-  if g is None:
-    static_q = torch.empty_like(xq)
-    static_q.copy_(xq)
-    side = torch.cuda.Stream(device=xq.device)
-    side.wait_stream(torch.cuda.current_stream())
-    with torch.cuda.stream(side):          # warm-up on the capture stream: workspaces, shared-memory attributes, NCCL channels
-      _run_sharded(index, static_q, k, id_offset, metric, process_group, gather, True)
-    torch.cuda.current_stream().wait_stream(side)
-    torch.cuda.synchronize()
-    torch.distributed.barrier(group=process_group)
-    graph = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(graph, capture_error_mode="thread_local"):
-      out, flag = _run_sharded(index, static_q, k, id_offset, metric, process_group, gather, True)
-    if len(graphs) >= 4:                   # a serving loop uses one or two shapes (full blocks and the tail block)
-      graphs.pop(next(iter(graphs)))
-    g = graphs[key] = (graph, static_q, out, flag)
-  graph, static_q, out, flag = g
-  static_q.copy_(xq)
-  graph.replay()
-  D, I = out[0].clone(), out[1].clone()     # the graph's own output buffers are overwritten by the next replay
-  return (D, I), int(flag.item()) != 0
 
 
 def _finish_sharded(got, nq, nqp, k, world, metric, process_group, gather, device):

@@ -586,7 +586,6 @@ def _trace_routes():
 @pytest.mark.gpu
 def test_routes_match_the_dispatcher(cd):
   env = dict(os.environ, CDML_TRACE="1")
-  env.pop("CDML_NO_RESB", None), env.pop("CDML_2CTA", None), env.pop("CDML_TMA_STORE", None)
   r = subprocess.run([sys.executable, os.path.abspath(__file__), "--trace-routes"], env=env, cwd=ROOT,
                      capture_output=True, text=True, timeout=900)
   assert r.returncode == 0 and "DONE" in r.stderr, r.stderr[-4000:]

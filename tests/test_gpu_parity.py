@@ -720,8 +720,16 @@ def test_mean_dist_matches_oracle(cd, golden):
 
 # ---------------------------------------------------------------- row M: in-batch semi-hard mining
 def test_semihard_mining_matches_oracle_up_to_fp16_selection_noise(cd):
+  _check_semihard_mining(cd, 700)                 # generic kernel
+
+
+def test_semihard_mining_resident_b_matches_oracle_up_to_fp16_selection_noise(cd):
+  _check_semihard_mining(cd, 2048)                # resident-B kernel (B >= 1024)
+
+
+def _check_semihard_mining(cd, B):
   rng = np.random.RandomState(11)
-  B, D, G = 700, 256, 400                       # few guids -> plenty of excluded (same-guid) candidates
+  D, G = 256, 4 * B // 7                        # few guids -> plenty of excluded (same-guid) candidates
   trip = O.synth_triplets(B, G, seed=3)
   base = O.l2_normalize(rng.standard_normal((G, D)))
   E = O.l2_normalize(base[trip.reshape(-1)] + 0.15 * rng.standard_normal((3 * B, D))).astype(np.float32)

@@ -279,7 +279,7 @@ def group_gemm_null():
         res.append(e0.elapsed_time(e1) / 5)
       ms = min(res)
       print("null M=%d N=%d K=%d epi=%d resb=%s: %.3f ms (runs %s)  %.1f TFLOP/s" %
-            (M, N, K, epi, "off" if os.environ.get("CDML_NO_RESB") else "on", ms, ["%.3f" % r for r in res], 2.0 * M * N * K / ms / 1e9), flush=True)
+            (M, N, K, epi, "on" if (not amn and not bmn and K <= 256 and M >= 1024) else "off", ms, ["%.3f" % r for r in res], 2.0 * M * N * K / ms / 1e9), flush=True)
 
 
 if __name__ == "__main__":
